@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- rendered messages/s of the NUTS message path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one pass of the hot path over one batch of synthetic input per rank:
@@ -68,6 +68,56 @@ def make_inputs(rank: int, n_msgs: int):
     ufile = synth.ban_file(1, N_BAN_ENTRIES, N_BAN_QUERIES, N_BAN_QUERIES, True, seed=seed)
     return dict(words=words, users=sh["users"], n_rooms=sh["n_rooms"], bodies=sh["bodies"], ops=sh["ops"],
                 speaker=sh["speaker"], sites=(st, so), names=(nt, no), sfile=sfile, ufile=ufile)
+
+
+DUMP_SEED = 0x333D
+DUMP_STREAM_CAP = 1 << 20           # bytes of a user's stream the sample looks at
+DUMP_HEAD_USERS = 8
+DUMP_POINTS = 2 << 20
+
+
+def dump_outputs(out_dir: str, lane: dict, dev) -> None:
+    """--dump-outputs: what one lane's last step handed its caller, as .npy files of float32 (bytes, 0/1 verdicts)
+    or float64 (offsets, counts), about 47 MB in all, so that two builds can be compared output for output.  The
+    three verdict arrays and the per-user stream offsets are written whole.  Of the ~5 GB of stream bytes, a sample
+    fixed by DUMP_SEED and the user count alone, so that it lines up element for element across builds whatever
+    stream lengths they produce: the first 1 MiB of the streams of 8 users (stream_heads, one row per user of
+    stream_head_users), and the bytes at 2M (user, offset < 1 MiB) pairs (stream_points).  -1 marks an offset at or
+    past the end of the user's stream."""
+    import torch
+
+    class DevBuf:                       # a buffer the library owns in HBM, seen by torch without a copy
+        def __init__(self, ptr, n, typestr):
+            self.__cuda_array_interface__ = dict(shape=(n,), typestr=typestr, data=(int(ptr), False), version=2)
+
+    s = lane["streams"]
+    n_users, total = int(s.n_users), int(s.total_bytes)
+    off = torch.as_tensor(DevBuf(s.off, n_users + 1, "<i8"), device=dev).cpu().numpy()
+    data = torch.as_tensor(DevBuf(s.bytes, total, "|u1"), device=dev) if total else torch.zeros(0, dtype=torch.uint8, device=dev)
+    lens = np.diff(off)
+    rng = np.random.default_rng(DUMP_SEED)
+    head_users = np.sort(rng.choice(n_users, min(DUMP_HEAD_USERS, n_users), replace=False))
+    heads = np.full((len(head_users), DUMP_STREAM_CAP), -1, np.float32)
+    for row, u in enumerate(head_users):
+        n = int(min(lens[u], DUMP_STREAM_CAP))
+        heads[row, :n] = data[int(off[u]):int(off[u]) + n].cpu().numpy()
+    pu = rng.integers(0, n_users, DUMP_POINTS)
+    pj = rng.integers(0, DUMP_STREAM_CAP, DUMP_POINTS)
+    inside = pj < lens[pu]
+    points = np.full(DUMP_POINTS, -1, np.float32)
+    points[inside] = data[torch.from_numpy(off[pu[inside]] + pj[inside]).to(dev)].cpu().numpy()
+    out = dict(contains_swearing=lane["verdict"].cpu().numpy().astype(np.float32),
+               site_banned=lane["vs"].cpu().numpy().astype(np.float32),
+               user_banned=lane["vu"].cpu().numpy().astype(np.float32),
+               stream_off=off.astype(np.float64),
+               n_deliveries=np.array([int(s.n_deliveries)], np.float64),
+               stream_head_users=head_users.astype(np.float64),
+               stream_heads=heads,
+               stream_points=points)
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, a in out.items():
+        np.save(d / f"{name}.npy", a)
 
 
 # ---------------------------------------------------------------------------------------
@@ -355,6 +405,7 @@ def run_ours(args):
         s = c.write_batch_dev(n_ops, d["text"].data_ptr(), d["off"].data_ptr(), d["kind"].data_ptr(),
                               d["target"].data_ptr(), d["exc"].data_ptr(), d["flags"].data_ptr(),
                               d["gate"].data_ptr(), L["verdict"].data_ptr())
+        L["streams"] = s
         t = c.timing()
         with state_lock:
             state["deliv"] += int(s.n_deliveries); state["bytes"] += int(s.total_bytes)
@@ -403,6 +454,8 @@ def run_ours(args):
     clk = clocks.stop()
     ms = e0.elapsed_time(e1)
     dev_state = dict(state)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, lanes[0], dev)
     # ---- per-kernel durations: the same step with every kernel on one stream (no k_render / k_direct beside
     #      the plan / the fan-out), so that each kernel is timed alone with CUDA events on its own stream
     ctx.set_overlap(False)
@@ -1002,7 +1055,13 @@ def main():
     ap.add_argument("--c5-chunk", type=int, default=10_000_000,
                     help="config 5: messages per GPU in one chunk = one write batch (default: the whole job in one; 1000000 = the same HBM per GPU at every N)")
     ap.add_argument("--c5-users", type=int, default=100_000)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (rank 0) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.config != "c3c4"):
+        ap.error("--dump-outputs is implemented for the default workload (--impl ours --config c3c4) only")
+    if args.dump_outputs and args.steps < 1:
+        ap.error("--dump-outputs writes the last timed step's results: it needs --steps 1 or more")
     if args.impl == "reference":
         return run_reference(args)
     if args.config != "c3c4":
