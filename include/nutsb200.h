@@ -165,8 +165,8 @@ int  nutsb_set_stream(nutsb_ctx *ctx, void *cuda_stream);
  * nutsb_set_users.  The queue tier then makes the relays: a room op naming a clone's room also queues
  * write_user(owner, "~FT[ <room> ]:~RS <str>") at the clone's place in the user list, unless the clone is
  * filtered like any recipient, hears nothing, its owner ignores everything, or (hear 1) the string does not
- * swear.  The batch tier takes ops as given: clones receive nothing there.  Room names: rm->name, default
- * "room<index>". */
+ * swear.  The host-buffer batch calls make them too; the device-buffer ones refuse the population (see
+ * nutsb_write_batch).  Room names: rm->name, default "room<index>". */
 int nutsb_set_clones(nutsb_ctx *ctx, int32_t n_users, const int32_t *owner, const uint8_t *hear);
 /* Remote users (nuts333.c:1299-1307): link[u] = index of the pseudo-user whose stream stands for the netlink
  * socket remote user u is reached through (a user in no room, flagged neither clone nor remote; several
@@ -219,8 +219,9 @@ int nutsb_set_users_remap(nutsb_ctx *ctx, int32_t n_users, int32_t n_rooms, cons
  * population (NUTSB_UF_CLONE / NUTSB_UF_REMOTE) the host-buffer calls (nutsb_write_batch, nutsb_write_batch_iov)
  * expand every op on the host exactly as the queue tier does -- the relays of nuts333.c:1416-1426 and the
  * MSG/EMSG frames of c:1299-1307, each under the op's own gate -- before the batch runs (needs an empty queue,
- * nutsb_set_clones / nutsb_set_remotes); the device-buffer calls (*_dev, nutsb_speech_batch*) take ops as they
- * are and return NUTSB_E_UNSUPPORTED for such a population rather than deliver different bytes. */
+ * nutsb_set_clones / nutsb_set_remotes); the device-buffer calls (*_dev, nutsb_write_batch_keep,
+ * nutsb_speech_batch*) take ops as they are and return NUTSB_E_UNSUPPORTED for such a population rather than
+ * deliver different bytes. */
 int nutsb_write_batch(nutsb_ctx *ctx, const nutsb_ops *ops, nutsb_streams *out);
 /* Device variant: every pointer in ops is a device pointer; streams stay in HBM.  The packed text is read
  * in aligned 16-byte vectors: it must be readable from the 16-byte boundary at or before its first byte to the

@@ -46,6 +46,53 @@ struct ClassSet {                    // one class granularity (with / without le
     i32 n_cls = 0, max_per_room = 0;
 };
 
+// An op list in host vectors (the queue; one shard's share of a routed batch).  The per-op vectors always
+// have one entry per op, so the op count and the text length mark a point to roll back to.
+struct HostOps {
+    std::vector<u8> text; std::vector<u64> off{0}; std::vector<u8> kind, flags;
+    std::vector<i32> target, except, gate;
+    struct Mark { size_t n, text; };
+
+    size_t n() const { return kind.size(); }
+    void push(u8 k, i32 t, const u8 *bytes, size_t len, i32 x, u8 f, i32 g)
+    {
+        text.insert(text.end(), bytes, bytes + len);
+        off.push_back((u64)text.size());
+        kind.push_back(k); target.push_back(t); except.push_back(x); flags.push_back(f); gate.push_back(g);
+    }
+    Mark mark() const { return { n(), text.size() }; }
+    void rollback(const Mark &m)
+    {
+        text.resize(m.text); off.resize(m.n + 1);
+        kind.resize(m.n); target.resize(m.n); except.resize(m.n); flags.resize(m.n); gate.resize(m.n);
+    }
+    void clear() { rollback({ 0, 0 }); }
+    // the list as a batch; gated only when given the verdicts its gates index
+    nutsb_ops view(const u8 *verdict) const
+    {
+        static const u8 z8 = 0; static const i32 z32 = 0;
+        nutsb_ops o{};
+        o.n_ops = (i64)n();
+        o.text = text.empty() ? &z8 : text.data(); o.text_off = off.data();
+        o.kind = kind.empty() ? &z8 : kind.data(); o.flags = flags.empty() ? &z8 : flags.data();
+        o.target = target.empty() ? &z32 : target.data(); o.except_user = except.empty() ? &z32 : except.data();
+        if (verdict) { o.gate = gate.empty() ? &z32 : gate.data(); o.verdict = verdict; }
+        return o;
+    }
+};
+
+// Profiling events (nutsb_set_profiling): the points a write batch records, one meaning each.
+enum Ev {
+    EV_START,                   // run_write begins
+    EV_RENDER0, EV_RENDER1,     // k_render
+    EV_DIRECT0, EV_DIRECT1,     // the direct ops: k_direct (nothing between the two when fused into the fan-out), k_direct_compact
+    EV_FAN0, EV_FAN1,           // the renderings to their recipients: k_fanout / k_fanout_direct, k_iov for gather lists
+    EV_END,                     // the batch's last kernel is done
+    EV_H2D0, EV_H2D1,           // the host input's copies to HBM
+    EV_D2H0, EV_D2H1,           // the result's copies to pinned host memory
+    EV_COUNT
+};
+
 struct nutsb_ctx {
     int device = 0;
     cudaStream_t stream = nullptr; bool own_stream = true;
@@ -56,7 +103,7 @@ struct nutsb_ctx {
     int sm_count = 148;
     std::string err;
     bool profiling = false; nutsb_timing tm{};
-    cudaEvent_t ev[12] = {};
+    cudaEvent_t ev[EV_COUNT] = {};
 
     // tables
     DBuf d_codetab;
@@ -109,8 +156,7 @@ struct nutsb_ctx {
     DBuf s_verb, s_speaker, s_body, s_boff;
 
     // queue tier
-    std::vector<u8> q_text; std::vector<u64> q_off{0}; std::vector<u8> q_kind, q_flags;
-    std::vector<i32> q_target, q_except, q_gate;
+    HostOps q;
     std::vector<u8> q_sw_text; std::vector<u64> q_sw_off{0};     // bodies whose swear verdict gates queued ops
     std::vector<u8> q_sw_verdict;                                // ... their verdicts, once taken (flush / review)
 
@@ -132,6 +178,13 @@ static int fail(nutsb_ctx *c, int code, const char *fmt, const char *a = "")
     return fail(c, e_ == cudaErrorMemoryAllocation ? NUTSB_E_NOMEM : NUTSB_E_CUDA, #call ": %s", cudaGetErrorString(e_)); } while (0)
 #define CKL() CK(cudaGetLastError())
 #define TRY(x) do { int r_ = (x); if (r_ != NUTSB_OK) return r_; } while (0)
+
+static int ev_record(nutsb_ctx *c, Ev e, cudaStream_t s)        // a profiling event, when profiling is on
+{
+    if (c->profiling) CK(cudaEventRecord(c->ev[e], s));
+    return NUTSB_OK;
+}
+static int ev_elapsed(nutsb_ctx *c, float *ms, Ev a, Ev b) { CK(cudaEventElapsedTime(ms, c->ev[a], c->ev[b])); return NUTSB_OK; }
 
 static int ensure(nutsb_ctx *c, DBuf &b, size_t bytes)
 {
@@ -651,7 +704,7 @@ static int set_users_impl(nutsb_ctx *c, int32_t n_users, int32_t n_rooms, const 
     }
     // queued ops name users and rooms by their index in the population they were queued under: a new
     // population may only come in between two flushes
-    if (!c->q_kind.empty() || !c->q_rec.empty())
+    if (c->q.n() || !c->q_rec.empty())
         return fail(c, NUTSB_E_STATE, "nutsb_set_users with ops still queued: flush first%s");
     c->have_users = false; c->have_streams = false;
     // review buffers live as long as their room / user does (the reference clears them in create_room c:2799,
@@ -765,6 +818,168 @@ struct IovReq {
     u64 slab_span = 0, direct_bytes = 0, n_iov = 0;      // h_out = the slab's two renderings, h_dir = the direct renderings
 };
 
+// What run_write's two tails take over from its steps A-E.
+struct Planned {
+    OpsView ops; PopView pop; ClassPrefix cpx; Sizes sz;
+    u32 *sv_slot, *counts; u64 *counters;
+    u64 off_base, slab_on, slab_off;
+    bool has_level, alias, par; cudaStream_t sd;
+};
+
+// The end of every write batch: the result (bytes = NULL: gather lists, no streams in HBM) and the byte counters.
+static void finish(nutsb_ctx *c, nutsb_streams *out, const u8 *bytes, u64 total, u64 deliveries,
+                   u64 slab, u64 fan_in, u64 fan_out, u64 render_in)
+{
+    c->last_total = total; c->have_streams = bytes != nullptr;      // (nutsb_stream_digests needs the streams)
+    c->tm.slab_bytes = slab; c->tm.fanout_bytes_in = fan_in; c->tm.fanout_bytes_out = fan_out; c->tm.render_bytes_in = render_in;
+    out->n_users = c->U; out->total_bytes = total; out->n_deliveries = deliveries;
+    out->off = c->d_off.as<u64>(); out->bytes = bytes; out->on_device = 1;
+}
+
+// Gather lists instead of streams: direct ops rendered one after the other (k_direct_compact), one list entry
+// per stretch of slab bytes and per direct rendering (k_iov); no copy plan, no fan-out.
+static int write_iov_tail(nutsb_ctx *c, const Planned &p, nutsb_streams *out, IovReq *iv)
+{
+    const i32 U = c->U; const Sizes &sz = p.sz;
+    cudaStream_t st = c->stream;
+    u32 *h32 = c->h_small.as<u32>(); u64 *h64 = c->h_small.as<u64>();
+    *iv = IovReq{ true, p.off_base + p.slab_off, sz.direct_bytes, 2ull * sz.n_events + (u64)U };
+    TRY(ensure(c, c->d_dir, sz.direct_bytes + 64));
+    TRY(ensure(c, c->d_iov, (size_t)iv->n_iov * sizeof(IovEnt)));
+    TRY(ensure(c, c->d_iov_first, (size_t)U * 8)); TRY(ensure(c, c->d_iov_cnt, (size_t)U * 4));
+    TRY(ensure_host(c, c->h_dir, (size_t)sz.direct_bytes + 64));                        // the entries hold host addresses
+    TRY(ensure_host(c, c->h_iov, (size_t)iv->n_iov * sizeof(IovEnt)));
+    TRY(ensure_host(c, c->h_iov_first, ((size_t)U + 1) * 8)); TRY(ensure_host(c, c->h_iov_cnt, ((size_t)U + 1) * 4));
+    TRY(ensure_host(c, c->h_off, ((size_t)U + 1) * 8));
+    TRY(ev_record(c, EV_DIRECT0, st));
+    if (sz.n_events > 0) {
+        DirectArgs da{ p.ops, p.pop, p.cpx, c->d_room_b_off.as<u32>(), c->d_ev_off.as<u32>(), c->d_sv_ukey.as<u32>(), c->d_sv_op.as<u32>(),
+                       c->d_sv_pre.as<u64>(), c->d_off.as<u64>(), p.sv_slot, c->d_sv_delta.as<i32>(), c->d_dir.as<u8>(), (i64)sz.n_events, p.counters,
+                       c->d_status.as<u32>(), c->d_slab.as<u8>(), p.off_base, 0u, c->d_slots.as<SlotInfo>(), c->d_dpre.as<u64>() };
+        NUTSB_LAUNCH_SMEM(cdiv(sz.n_events, NUTSB_DIRECT_THREADS), NUTSB_DIRECT_THREADS, NUTSB_DIR_SMEM, st, k_direct_compact, da); CKL();
+        c->tm.launches++;
+    }
+    TRY(ev_record(c, EV_DIRECT1, st)); TRY(ev_record(c, EV_FAN0, st));
+    IovArgs ia{ p.pop, c->d_slots.as<SlotInfo>(), c->d_vp_on.as<u64>(), c->d_vp_off.as<u64>(), c->d_sv_ukey.as<u32>(), p.sv_slot,
+                c->d_dpre.as<u64>(), sz.n_events, (u64)(size_t)c->h_out.p, (u64)(size_t)c->h_dir.p, p.off_base,
+                c->d_iov.as<IovEnt>(), c->d_iov_first.as<u64>(), c->d_iov_cnt.as<u32>(), p.counters };
+    NUTSB_LAUNCH(cdiv(std::max<u64>(sz.n_events, (u64)U), 256), 256, st, k_iov, ia); CKL();
+    c->tm.launches++;
+    TRY(ev_record(c, EV_FAN1, st)); TRY(ev_record(c, EV_END, st));
+    // the rest of the result, beside the slab's copy on the side stream
+    if (sz.direct_bytes) CK(cudaMemcpyAsync(c->h_dir.p, c->d_dir.p, (size_t)sz.direct_bytes, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(c->h_iov.p, c->d_iov.p, (size_t)iv->n_iov * sizeof(IovEnt), cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(c->h_iov_first.p, c->d_iov_first.p, (size_t)U * 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(c->h_iov_cnt.p, c->d_iov_cnt.p, (size_t)U * 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(c->h_off.p, c->d_off.p, ((size_t)U + 1) * 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(h64 + 8, p.counters, 24, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(h32 + 4, c->d_status.p, 4, cudaMemcpyDeviceToHost, st));
+    if (p.par) CK(cudaStreamWaitEvent(st, c->dep[1], 0));      // the slab is rendered and on the host
+    TRY(ev_record(c, EV_D2H1, st));
+    CK(cudaStreamSynchronize(st));
+    TRY(status_to_error(c, h32[4]));
+    if (c->profiling) {
+        TRY(ev_elapsed(c, &c->tm.plan_ms, EV_START, EV_DIRECT0));
+        TRY(ev_elapsed(c, &c->tm.render_ms, EV_RENDER0, EV_RENDER1));
+        TRY(ev_elapsed(c, &c->tm.fanout_ms, EV_FAN0, EV_FAN1));
+        TRY(ev_elapsed(c, &c->tm.direct_ms, EV_DIRECT0, EV_DIRECT1));
+        TRY(ev_elapsed(c, &c->tm.total_ms, EV_START, EV_END));
+        TRY(ev_elapsed(c, &c->tm.d2h_ms, EV_END, EV_D2H1));        // what of the copies is left after the last kernel
+    }
+    finish(c, out, nullptr, sz.total_bytes, h64[8], p.slab_on + p.slab_off, 0, 0, h64[10]);
+    return NUTSB_OK;
+}
+
+static int write_streams_tail(nutsb_ctx *c, const Planned &p, nutsb_streams *out)
+{
+    const Sizes &sz = p.sz;
+    cudaStream_t st = c->stream, sd = p.sd;
+    u32 *h32 = c->h_small.as<u32>(); u64 *h64 = c->h_small.as<u64>();
+    TRY(ensure(c, c->d_out, sz.total_bytes + 64));
+    Geometry geo{ c->d_room_b_off.as<u32>(), c->d_room_tile_off.as<u32>(), c->d_room_cell_off.as<u64>(), c->d_room_item_off.as<u32>() };
+
+    // -- I. direct ops + seams.  With the overlap on they share ONE launch with the fan-out (k_fanout_direct,
+    //    below): blocks of both kinds on every SM.  Otherwise (or when there is nothing to fan out) k_direct
+    //    runs by itself, here.
+    const bool fan = sz.cells > 0 && sz.items > 0;
+    const bool fused = p.par && fan && sz.n_events > 0;
+    DirectArgs da{ p.ops, p.pop, p.cpx, c->d_room_b_off.as<u32>(), c->d_ev_off.as<u32>(), c->d_sv_ukey.as<u32>(), c->d_sv_op.as<u32>(),
+                   c->d_sv_pre.as<u64>(), c->d_off.as<u64>(), p.sv_slot, c->d_sv_delta.as<i32>(), c->d_out.as<u8>(), (i64)sz.n_events, p.counters,
+                   c->d_status.as<u32>(), c->d_slab.as<u8>(), p.off_base, p.has_level ? 1u : 0u, c->d_slots.as<SlotInfo>(), nullptr };
+    u32 n_dir = cdiv(sz.n_events, NUTSB_DIRECT_THREADS);
+    if (fused && c->fd_dir_per_sm > 0) n_dir = std::min(n_dir, (u32)(c->sm_count * c->fd_dir_per_sm));   // grid-strided direct blocks
+    TRY(ev_record(c, EV_DIRECT0, sd));
+    if (sz.n_events > 0 && !fused) {
+        if (p.par) { CK(cudaEventRecord(c->dep[2], st)); CK(cudaStreamWaitEvent(sd, c->dep[2], 0)); }
+        NUTSB_LAUNCH_SMEM(n_dir, NUTSB_DIRECT_THREADS, NUTSB_DIR_SMEM, sd, k_direct, da); CKL();
+        c->tm.launches++;
+    }
+    TRY(ev_record(c, EV_DIRECT1, sd));
+    if (p.par) CK(cudaEventRecord(c->dep[3], sd));
+
+    // -- F. copy plan: the run list and the work-item descriptors
+    if (fan) {
+        TRY(ensure(c, c->d_items, (size_t)sz.items * sizeof(ItemDesc)));
+        u32 *cursor = p.counts + 4;
+        CK(cudaMemsetAsync(cursor, 0, 4, st));
+        PlanArgs pa{ p.pop, geo, p.cpx, c->d_off.as<u64>(), c->d_ev_off.as<u32>(), c->d_sv_ukey.as<u32>(), c->d_sv_delta.as<i32>(),
+                     c->d_sv_pre.as<u64>(), c->d_bl_meta.as<u32>(), (u64)sz.cells, p.off_base, p.has_level ? 1u : 0u,
+                     c->d_slots.as<SlotInfo>(), cursor, nullptr, c->d_items.as<ItemDesc>(), p.counters, c->d_status.as<u32>() };
+        // plain listeners: at most one run per cell plus one per event; behind a filter the count is taken first
+        u64 n_runs = sz.cells + sz.n_events;
+        if (!p.alias) {
+            NUTSB_LAUNCH(sz.items, NUTSB_UCHUNK, st, k_plan<false>, pa); CKL();
+            CK(cudaMemcpyAsync(h32 + 6, cursor, 4, cudaMemcpyDeviceToHost, st));
+            CK(cudaMemsetAsync(cursor, 0, 4, st));
+            CK(cudaStreamSynchronize(st));
+            n_runs = h32[6];
+            c->tm.launches++;
+        }
+        if (n_runs >= 0xfffffff0ull) return fail(c, NUTSB_E_RANGE, "more than 2^32 copy runs in one batch%s");
+        TRY(ensure(c, c->d_runs, (n_runs + 1) * sizeof(uint4)));
+        pa.runs = c->d_runs.as<uint4>();
+        NUTSB_LAUNCH(sz.items, NUTSB_UCHUNK, st, k_plan<true>, pa); CKL();
+        c->tm.launches++;
+    }
+
+    // -- H. fan-out: after the slab is rendered
+    if (p.par) CK(cudaStreamWaitEvent(st, c->dep[1], 0));
+    TRY(ev_record(c, EV_FAN0, st));
+    if (fan) {
+        FanoutArgs fa{ c->d_items.as<ItemDesc>(), c->d_runs.as<uint4>(), c->d_slab.as<u8>(), p.off_base, c->d_out.as<u8>() };
+        if (fused) {
+            const u32 total = sz.items + n_dir;
+            const u32 stride = std::max(1u, total / n_dir);        // a direct block every `stride` blocks
+            NUTSB_LAUNCH_SMEM(total, NUTSB_FAN_THREADS, NUTSB_FD_SMEM, st, k_fanout_direct, fa, da, n_dir, stride); CKL();
+        } else {
+            NUTSB_LAUNCH_SMEM(sz.items, NUTSB_FAN_THREADS, NUTSB_FAN_SMEM, st, k_fanout, fa); CKL();
+        }
+        c->tm.launches++; c->tm.fanout_launches = 1;
+    }
+    TRY(ev_record(c, EV_FAN1, st));
+    if (p.par) CK(cudaStreamWaitEvent(st, c->dep[3], 0));
+    TRY(ev_record(c, EV_END, st));
+
+    NUTSB_LAUNCH(1, 32, st, k_readback_end, p.counters, c->d_status.as<u32>(), h64 + 8, h32 + 4); CKL();
+    c->tm.launches++;
+    CK(cudaStreamSynchronize(st));
+    TRY(status_to_error(c, h32[4]));
+    c->last.valid = true; c->last.ops = p.ops; c->last.cpx = p.cpx; c->last.has_level = p.has_level; c->last.off_base = p.off_base; c->last.sv_slot = p.sv_slot;
+    if (c->profiling) {
+        // with the side stream on, render_ms / direct_ms are the side kernels' own spans and overlap plan_ms / fanout_ms
+        CK(cudaEventSynchronize(c->ev[EV_DIRECT1]));
+        TRY(ev_elapsed(c, &c->tm.plan_ms, EV_START, EV_FAN0));
+        TRY(ev_elapsed(c, &c->tm.render_ms, EV_RENDER0, EV_RENDER1));
+        TRY(ev_elapsed(c, &c->tm.fanout_ms, EV_FAN0, EV_FAN1));
+        TRY(ev_elapsed(c, &c->tm.direct_ms, EV_DIRECT0, EV_DIRECT1));
+        TRY(ev_elapsed(c, &c->tm.total_ms, EV_START, EV_END));
+        if (!p.par) c->tm.plan_ms -= c->tm.render_ms + c->tm.direct_ms;
+    }
+    const u64 slab = p.slab_on + p.slab_off;                   // (fan-out input: each rendering of a tile is read once per work item)
+    finish(c, out, c->d_out.as<u8>(), sz.total_bytes, h64[8], slab, slab, sz.total_bytes - h64[9], h64[10]);
+    return NUTSB_OK;
+}
+
 static int run_write(nutsb_ctx *c, const nutsb_ops *o, nutsb_streams *out, IovReq *iv = nullptr)
 {
     if (!c->have_users) return fail(c, NUTSB_E_STATE, "nutsb_set_users has not been called%s");
@@ -774,7 +989,7 @@ static int run_write(nutsb_ctx *c, const nutsb_ops *o, nutsb_streams *out, IovRe
     c->have_streams = false; c->last.valid = false;
     c->tm.launches = 0; c->tm.fanout_launches = 0;
     if (c->side) CK(cudaStreamSynchronize(c->side));           // idle unless an earlier batch failed half-way
-    if (c->profiling) CK(cudaEventRecord(c->ev[0], st));
+    TRY(ev_record(c, EV_START, st));
 
     TRY(ensure(c, c->d_off, ((size_t)U + 1) * 8));
     u32 *h32 = c->h_small.as<u32>(); u64 *h64 = c->h_small.as<u64>();
@@ -782,12 +997,8 @@ static int run_write(nutsb_ctx *c, const nutsb_ops *o, nutsb_streams *out, IovRe
     auto finish_empty = [&]() -> int {
         CK(cudaMemsetAsync(c->d_off.p, 0, ((size_t)U + 1) * 8, st));
         TRY(ensure(c, c->d_out, 16));
-        if (c->profiling) { for (int q = 1; q < 4; ++q) CK(cudaEventRecord(c->ev[q], st)); }
         CK(cudaStreamSynchronize(st));
-        c->last_total = 0; c->have_streams = true;
-        c->tm.fanout_bytes_in = c->tm.fanout_bytes_out = 0; c->tm.slab_bytes = c->tm.render_bytes_in = 0;
-        out->n_users = U; out->total_bytes = 0; out->n_deliveries = 0;
-        out->off = c->d_off.as<u64>(); out->bytes = c->d_out.as<u8>(); out->on_device = 1;
+        finish(c, out, c->d_out.as<u8>(), 0, 0, 0, 0, 0, 0);
         return NUTSB_OK;
     };
     if (n == 0) return finish_empty();
@@ -897,9 +1108,8 @@ static int run_write(nutsb_ctx *c, const nutsb_ops *o, nutsb_streams *out, IovRe
     if (off_base + slab_off >= (1ull << 40)) return fail(c, NUTSB_E_RANGE, "more than 2^40 bytes of rendered slab in one batch%s");
     TRY(ensure(c, c->d_slab, off_base + slab_off + 256));
     if (compact) TRY(ensure_host(c, c->h_out, (size_t)(off_base + slab_off) + 64));      // before anything is queued on the side stream
-    c->tm.slab_bytes = slab_on + slab_off;
     if (par) { CK(cudaEventRecord(c->dep[0], st)); CK(cudaStreamWaitEvent(sd, c->dep[0], 0)); }
-    if (c->profiling) CK(cudaEventRecord(c->ev[1], sd));
+    TRY(ev_record(c, EV_RENDER0, sd));
     {
         RenderArgs ra{ ops, c->d_codetab.as<u8>(), c->d_bl_op.as<u32>(), c->d_vp_on.as<u64>(), c->d_vp_off.as<u64>(), counts,
                        c->d_slab.as<u8>(), off_base, counters, c->d_status.as<u32>() };
@@ -909,7 +1119,7 @@ static int run_write(nutsb_ctx *c, const nutsb_ops *o, nutsb_streams *out, IovRe
         NUTSB_LAUNCH(grid, NUTSB_REN_THREADS, sd, k_render, ra); CKL();
         c->tm.launches++;
     }
-    if (c->profiling) CK(cudaEventRecord(c->ev[8], sd));
+    TRY(ev_record(c, EV_RENDER1, sd));
     // gather lists: the slab is part of the result as it stands -- on its way to the host while the planning goes on
     if (compact && off_base + slab_off) CK(cudaMemcpyAsync(c->h_out.p, c->d_slab.p, (size_t)(off_base + slab_off), cudaMemcpyDeviceToHost, sd));
     if (par) CK(cudaEventRecord(c->dep[1], sd));
@@ -950,178 +1160,45 @@ static int run_write(nutsb_ctx *c, const nutsb_ops *o, nutsb_streams *out, IovRe
                  compact ? c->d_dpre.as<u64>() : (const u64 *)nullptr); CKL();
     c->tm.launches++;
     CK(cudaStreamSynchronize(st));
-    const Sizes sz = *hs;
-    if (sz.slab_on != slab_on || sz.slab_off != slab_off) return fail(c, NUTSB_E_CUDA, "internal: slab size mismatch%s");
-    if (compact) {
-        // -- gather lists instead of streams: direct ops rendered one after the other (k_direct_compact), one
-        //    list entry per stretch of slab bytes and per direct rendering (k_iov); no copy plan, no fan-out
-        iv->compact = true;
-        iv->slab_span = off_base + slab_off;
-        iv->direct_bytes = sz.direct_bytes;
-        iv->n_iov = 2ull * sz.n_events + (u64)U;
-        TRY(ensure(c, c->d_dir, sz.direct_bytes + 64));
-        TRY(ensure(c, c->d_iov, (size_t)iv->n_iov * sizeof(IovEnt)));
-        TRY(ensure(c, c->d_iov_first, (size_t)U * 8)); TRY(ensure(c, c->d_iov_cnt, (size_t)U * 4));
-        TRY(ensure_host(c, c->h_dir, (size_t)sz.direct_bytes + 64));                        // the entries hold host addresses
-        TRY(ensure_host(c, c->h_iov, (size_t)iv->n_iov * sizeof(IovEnt)));
-        TRY(ensure_host(c, c->h_iov_first, ((size_t)U + 1) * 8)); TRY(ensure_host(c, c->h_iov_cnt, ((size_t)U + 1) * 4));
-        TRY(ensure_host(c, c->h_off, ((size_t)U + 1) * 8));
-        if (c->profiling) { CK(cudaEventRecord(c->ev[9], st)); }
-        if (sz.n_events > 0) {
-            DirectArgs da{ ops, pop, cpx, c->d_room_b_off.as<u32>(), c->d_ev_off.as<u32>(), c->d_sv_ukey.as<u32>(), c->d_sv_op.as<u32>(),
-                           c->d_sv_pre.as<u64>(), c->d_off.as<u64>(), sv_slot, c->d_sv_delta.as<i32>(), c->d_dir.as<u8>(), (i64)sz.n_events, counters,
-                           c->d_status.as<u32>(), c->d_slab.as<u8>(), off_base, 0u, c->d_slots.as<SlotInfo>(), c->d_dpre.as<u64>() };
-            NUTSB_LAUNCH_SMEM(cdiv(sz.n_events, NUTSB_DIRECT_THREADS), NUTSB_DIRECT_THREADS, NUTSB_DIR_SMEM, st, k_direct_compact, da); CKL();
-            c->tm.launches++;
-        }
-        if (c->profiling) { CK(cudaEventRecord(c->ev[3], st)); CK(cudaEventRecord(c->ev[10], st)); }
-        IovArgs ia{ pop, c->d_slots.as<SlotInfo>(), c->d_vp_on.as<u64>(), c->d_vp_off.as<u64>(), c->d_sv_ukey.as<u32>(), sv_slot,
-                    c->d_dpre.as<u64>(), sz.n_events, (u64)(size_t)c->h_out.p, (u64)(size_t)c->h_dir.p, off_base,
-                    c->d_iov.as<IovEnt>(), c->d_iov_first.as<u64>(), c->d_iov_cnt.as<u32>(), counters };
-        NUTSB_LAUNCH(cdiv(std::max<u64>(sz.n_events, (u64)U), 256), 256, st, k_iov, ia); CKL();
-        c->tm.launches++;
-        if (c->profiling) { CK(cudaEventRecord(c->ev[2], st)); CK(cudaEventRecord(c->ev[11], st)); }
-        // the rest of the result, beside the slab's copy on the side stream
-        if (sz.direct_bytes) CK(cudaMemcpyAsync(c->h_dir.p, c->d_dir.p, (size_t)sz.direct_bytes, cudaMemcpyDeviceToHost, st));
-        CK(cudaMemcpyAsync(c->h_iov.p, c->d_iov.p, (size_t)iv->n_iov * sizeof(IovEnt), cudaMemcpyDeviceToHost, st));
-        CK(cudaMemcpyAsync(c->h_iov_first.p, c->d_iov_first.p, (size_t)U * 8, cudaMemcpyDeviceToHost, st));
-        CK(cudaMemcpyAsync(c->h_iov_cnt.p, c->d_iov_cnt.p, (size_t)U * 4, cudaMemcpyDeviceToHost, st));
-        CK(cudaMemcpyAsync(c->h_off.p, c->d_off.p, ((size_t)U + 1) * 8, cudaMemcpyDeviceToHost, st));
-        CK(cudaMemcpyAsync(h64 + 8, counters, 24, cudaMemcpyDeviceToHost, st));
-        CK(cudaMemcpyAsync(h32 + 4, c->d_status.p, 4, cudaMemcpyDeviceToHost, st));
-        if (par) CK(cudaStreamWaitEvent(st, c->dep[1], 0));    // the slab is rendered and on the host
-        if (c->profiling) CK(cudaEventRecord(c->ev[6], st));
-        CK(cudaStreamSynchronize(st));
-        TRY(status_to_error(c, h32[4]));
-        c->last_total = sz.total_bytes; c->have_streams = false;     // no streams in HBM (nutsb_stream_digests needs them)
-        if (c->profiling) {
-            CK(cudaEventElapsedTime(&c->tm.plan_ms, c->ev[0], c->ev[9]));
-            CK(cudaEventElapsedTime(&c->tm.render_ms, c->ev[1], c->ev[8]));
-            CK(cudaEventElapsedTime(&c->tm.fanout_ms, c->ev[10], c->ev[2]));
-            CK(cudaEventElapsedTime(&c->tm.direct_ms, c->ev[9], c->ev[3]));
-            CK(cudaEventElapsedTime(&c->tm.total_ms, c->ev[0], c->ev[11]));
-            CK(cudaEventElapsedTime(&c->tm.d2h_ms, c->ev[11], c->ev[6]));      // what of the copies is left after the last kernel
-        }
-        c->tm.fanout_bytes_out = 0; c->tm.fanout_bytes_in = 0; c->tm.render_bytes_in = h64[10];
-        out->n_users = U; out->total_bytes = sz.total_bytes; out->n_deliveries = h64[8];
-        out->off = c->d_off.as<u64>(); out->bytes = nullptr; out->on_device = 1;
-        return NUTSB_OK;
-    }
-    TRY(ensure(c, c->d_out, sz.total_bytes + 64));
-    Geometry geo{ c->d_room_b_off.as<u32>(), c->d_room_tile_off.as<u32>(), c->d_room_cell_off.as<u64>(), c->d_room_item_off.as<u32>() };
-    c->tm.fanout_launches = 0;
-
-    // -- I. direct ops + seams.  With the overlap on they share ONE launch with the fan-out (k_fanout_direct,
-    //    below): blocks of both kinds on every SM.  Otherwise (or when there is nothing to fan out) k_direct
-    //    runs by itself, here.
-    const bool fan = sz.cells > 0 && sz.items > 0;
-    const bool fused = par && fan && sz.n_events > 0;
-    DirectArgs da{ ops, pop, cpx, c->d_room_b_off.as<u32>(), c->d_ev_off.as<u32>(), c->d_sv_ukey.as<u32>(), c->d_sv_op.as<u32>(),
-                   c->d_sv_pre.as<u64>(), c->d_off.as<u64>(), sv_slot, c->d_sv_delta.as<i32>(), c->d_out.as<u8>(), (i64)sz.n_events, counters,
-                   c->d_status.as<u32>(), c->d_slab.as<u8>(), off_base, has_level ? 1u : 0u, c->d_slots.as<SlotInfo>(), nullptr };
-    u32 n_dir = cdiv(sz.n_events, NUTSB_DIRECT_THREADS);
-    if (fused && c->fd_dir_per_sm > 0) n_dir = std::min(n_dir, (u32)(c->sm_count * c->fd_dir_per_sm));   // grid-strided direct blocks
-    if (c->profiling) CK(cudaEventRecord(c->ev[9], sd));
-    if (sz.n_events > 0 && !fused) {
-        if (par) { CK(cudaEventRecord(c->dep[2], st)); CK(cudaStreamWaitEvent(sd, c->dep[2], 0)); }
-        NUTSB_LAUNCH_SMEM(n_dir, NUTSB_DIRECT_THREADS, NUTSB_DIR_SMEM, sd, k_direct, da); CKL();
-        c->tm.launches++;
-    }
-    if (c->profiling) CK(cudaEventRecord(c->ev[3], sd));
-    if (par) CK(cudaEventRecord(c->dep[3], sd));
-
-    // -- F. copy plan: the run list and the work-item descriptors
-    if (fan) {
-        TRY(ensure(c, c->d_items, (size_t)sz.items * sizeof(ItemDesc)));
-        u32 *cursor = counts + 4;
-        CK(cudaMemsetAsync(cursor, 0, 4, st));
-        PlanArgs pa{ pop, geo, cpx, c->d_off.as<u64>(), c->d_ev_off.as<u32>(), c->d_sv_ukey.as<u32>(), c->d_sv_delta.as<i32>(),
-                     c->d_sv_pre.as<u64>(), c->d_bl_meta.as<u32>(), (u64)sz.cells, off_base, has_level ? 1u : 0u,
-                     c->d_slots.as<SlotInfo>(), cursor, nullptr, c->d_items.as<ItemDesc>(), counters, c->d_status.as<u32>() };
-        // plain listeners: at most one run per cell plus one per event; behind a filter the count is taken first
-        u64 n_runs = sz.cells + sz.n_events;
-        if (!alias) {
-            NUTSB_LAUNCH(sz.items, NUTSB_UCHUNK, st, k_plan<false>, pa); CKL();
-            CK(cudaMemcpyAsync(h32 + 6, cursor, 4, cudaMemcpyDeviceToHost, st));
-            CK(cudaMemsetAsync(cursor, 0, 4, st));
-            CK(cudaStreamSynchronize(st));
-            n_runs = h32[6];
-            c->tm.launches++;
-        }
-        if (n_runs >= 0xfffffff0ull) return fail(c, NUTSB_E_RANGE, "more than 2^32 copy runs in one batch%s");
-        TRY(ensure(c, c->d_runs, (n_runs + 1) * sizeof(uint4)));
-        pa.runs = c->d_runs.as<uint4>();
-        NUTSB_LAUNCH(sz.items, NUTSB_UCHUNK, st, k_plan<true>, pa); CKL();
-        c->tm.launches++;
-    }
-
-    // -- H. fan-out: after the slab is rendered
-    if (par) CK(cudaStreamWaitEvent(st, c->dep[1], 0));
-    if (c->profiling) CK(cudaEventRecord(c->ev[10], st));
-    if (fan) {
-        FanoutArgs fa{ c->d_items.as<ItemDesc>(), c->d_runs.as<uint4>(), c->d_slab.as<u8>(), off_base, c->d_out.as<u8>() };
-        if (fused) {
-            const u32 total = sz.items + n_dir;
-            const u32 stride = std::max(1u, total / n_dir);        // a direct block every `stride` blocks
-            NUTSB_LAUNCH_SMEM(total, NUTSB_FAN_THREADS, NUTSB_FD_SMEM, st, k_fanout_direct, fa, da, n_dir, stride); CKL();
-        } else {
-            NUTSB_LAUNCH_SMEM(sz.items, NUTSB_FAN_THREADS, NUTSB_FAN_SMEM, st, k_fanout, fa); CKL();
-        }
-        c->tm.launches++; c->tm.fanout_launches = 1;
-    }
-    if (c->profiling) CK(cudaEventRecord(c->ev[2], st));
-    if (par) CK(cudaStreamWaitEvent(st, c->dep[3], 0));
-    if (c->profiling) CK(cudaEventRecord(c->ev[11], st));
-
-    NUTSB_LAUNCH(1, 32, st, k_readback_end, counters, c->d_status.as<u32>(), h64 + 8, h32 + 4); CKL();
-    c->tm.launches++;
-    CK(cudaStreamSynchronize(st));
-    TRY(status_to_error(c, h32[4]));
-    c->last_total = sz.total_bytes; c->have_streams = true;
-    c->last.valid = true; c->last.ops = ops; c->last.cpx = cpx; c->last.has_level = has_level; c->last.off_base = off_base; c->last.sv_slot = sv_slot;
-    if (c->profiling) {
-        // with the side stream on, render_ms / direct_ms are the side kernels' own spans and overlap plan_ms / fanout_ms
-        CK(cudaEventSynchronize(c->ev[3]));
-        CK(cudaEventElapsedTime(&c->tm.plan_ms, c->ev[0], c->ev[10]));
-        CK(cudaEventElapsedTime(&c->tm.render_ms, c->ev[1], c->ev[8]));
-        CK(cudaEventElapsedTime(&c->tm.fanout_ms, c->ev[10], c->ev[2]));
-        CK(cudaEventElapsedTime(&c->tm.direct_ms, c->ev[9], c->ev[3]));
-        CK(cudaEventElapsedTime(&c->tm.total_ms, c->ev[0], c->ev[11]));
-        if (!par) c->tm.plan_ms -= c->tm.render_ms + c->tm.direct_ms;
-    }
-    c->tm.fanout_bytes_out = sz.total_bytes - h64[9];
-    c->tm.fanout_bytes_in = c->tm.slab_bytes;          // each rendering of a tile is read once per work item
-    c->tm.render_bytes_in = h64[10];
-    out->n_users = U; out->total_bytes = sz.total_bytes; out->n_deliveries = h64[8];
-    out->off = c->d_off.as<u64>(); out->bytes = c->d_out.as<u8>(); out->on_device = 1;
-    return NUTSB_OK;
+    const Planned p{ ops, pop, cpx, *hs, sv_slot, counts, counters, off_base, slab_on, slab_off, has_level, alias, par, sd };
+    if (p.sz.slab_on != slab_on || p.sz.slab_off != slab_off) return fail(c, NUTSB_E_CUDA, "internal: slab size mismatch%s");
+    return compact ? write_iov_tail(c, p, out, iv) : write_streams_tail(c, p, out);
 }
 
-static int check_ops(nutsb_ctx *c, const nutsb_ops *o, nutsb_streams *out)
+static int check_ops(nutsb_ctx *c, const nutsb_ops *o)
 {
-    if (!c || !o || !out || o->n_ops < 0) return fail(c, NUTSB_E_INVAL, "null argument or negative n_ops%s");
+    if (!c || !o || o->n_ops < 0) return fail(c, NUTSB_E_INVAL, "null argument or negative n_ops%s");
     if (o->n_ops >= 0xfffffff0ll) return fail(c, NUTSB_E_RANGE, "more than 2^32 ops in one batch%s");
     if (o->n_ops && (!o->text_off || !o->kind || !o->target || !o->except_user || !o->flags))
         return fail(c, NUTSB_E_INVAL, "ops array is NULL%s");
     return NUTSB_OK;
 }
 
-// Clones and remote users (nuts333.c:1416-1426, 1299-1307) are reached through relays / frames that are
-// extra write_user calls, made on the host (q_push).  The device tiers take ops as they are, so with such
-// users in the population they refuse rather than deliver something else than the reference would.
-static int no_relays_on_device(nutsb_ctx *c)
+// The host-side check of op i, for the paths that expand or route ops on the host before the device sees
+// them: NUTSB_OK, or the error code with *why set.
+static int host_op_error(const nutsb_ops *o, i64 i, i32 U, i32 R, const char **why)
 {
-    if (c && c->has_clones)
-        return fail(c, NUTSB_E_UNSUPPORTED, "population holds clones / remote users: use the host-buffer or the queue tier%s");
+    if (o->text_off[i + 1] < o->text_off[i]) { *why = "text_off is not monotone"; return NUTSB_E_INVAL; }
+    const u8 k = o->kind[i];
+    if (k == NUTSB_OP_NONE) return NUTSB_OK;
+    if (k > NUTSB_OP_LEVEL) { *why = "unknown op kind"; return NUTSB_E_INVAL; }
+    const i32 t = o->target[i], x = o->except_user[i];
+    if (x >= U || x < -1 || (k == NUTSB_OP_USER && t >= U) || (k == NUTSB_OP_ROOM && (t >= R || t < -1))) {
+        *why = "user/room index out of range"; return NUTSB_E_RANGE;
+    }
     return NUTSB_OK;
 }
 
-NUTSB_API int nutsb_write_batch_dev(nutsb_ctx *c, const nutsb_ops *o, nutsb_streams *out)
+// Clones and remote users (nuts333.c:1416-1426, 1299-1307) are reached through relays / frames that are
+// extra write_user calls, made on the host (q_push).  Ops that have not been through that expansion are
+// refused with such users in the population, rather than delivered differently from the reference.
+// Every write entry point starts here.
+static int begin_write(nutsb_ctx *c, bool expanded)
 {
-    TRY(check_ops(c, o, out));
-    TRY(no_relays_on_device(c));
+    if (!expanded && c->has_clones)
+        return fail(c, NUTSB_E_UNSUPPORTED, "population holds clones / remote users: use the host-buffer or the queue tier%s");
     CK(cudaSetDevice(c->device));
-    return run_write(c, o, out);
+    return NUTSB_OK;
 }
 
 // ops in host memory -> the context's staging buffers in HBM (*d = the same batch with device pointers)
@@ -1129,8 +1206,9 @@ static int upload_ops(nutsb_ctx *c, const nutsb_ops *o, nutsb_ops *d)
 {
     const i64 n = o->n_ops;
     cudaStream_t st = c->stream;
+    TRY(ev_record(c, EV_H2D0, st));
     *d = *o;
-    if (n <= 0) return NUTSB_OK;
+    if (n <= 0) return ev_record(c, EV_H2D1, st);
     const u64 t0 = o->text_off[0], t1 = o->text_off[n];
     if (t1 < t0) return fail(c, NUTSB_E_INVAL, "text_off is not monotone%s");
     if (t1 > t0 && !o->text) return fail(c, NUTSB_E_INVAL, "text is NULL%s");
@@ -1151,90 +1229,93 @@ static int upload_ops(nutsb_ctx *c, const nutsb_ops *o, nutsb_ops *d)
         TRY(upload(c, c->s_verdict, o->verdict, (size_t)(mx + 1)));
         d->gate = c->s_gate.as<i32>(); d->verdict = c->s_verdict.as<u8>();
     }
-    return NUTSB_OK;
+    return ev_record(c, EV_H2D1, st);
 }
 
-// ops in host memory, streams back in pinned host memory; the ops are taken as they are
-static int write_batch_host(nutsb_ctx *c, const nutsb_ops *o, nutsb_streams *out)
+// Streams HBM -> pinned host memory (h_off, h_out)
+static int streams_to_host(nutsb_ctx *c, const nutsb_streams &ds)
 {
-    TRY(check_ops(c, o, out));
-    CK(cudaSetDevice(c->device));
     cudaStream_t st = c->stream;
-    if (c->profiling) CK(cudaEventRecord(c->ev[4], st));
-    nutsb_ops d;
-    TRY(upload_ops(c, o, &d));
-    if (c->profiling) CK(cudaEventRecord(c->ev[5], st));
-    nutsb_streams ds{};
-    TRY(run_write(c, &d, &ds));
-    if (c->profiling) { CK(cudaEventElapsedTime(&c->tm.h2d_ms, c->ev[4], c->ev[5])); CK(cudaEventRecord(c->ev[4], st)); }
+    TRY(ev_record(c, EV_D2H0, st));
     TRY(ensure_host(c, c->h_off, ((size_t)c->U + 1) * 8));
     TRY(ensure_host(c, c->h_out, (size_t)ds.total_bytes + 16));
     CK(cudaMemcpyAsync(c->h_off.p, ds.off, ((size_t)c->U + 1) * 8, cudaMemcpyDeviceToHost, st));
     if (ds.total_bytes) CK(cudaMemcpyAsync(c->h_out.p, ds.bytes, (size_t)ds.total_bytes, cudaMemcpyDeviceToHost, st));
-    if (c->profiling) CK(cudaEventRecord(c->ev[5], st));
+    TRY(ev_record(c, EV_D2H1, st));
     CK(cudaStreamSynchronize(st));
-    if (c->profiling) CK(cudaEventElapsedTime(&c->tm.d2h_ms, c->ev[4], c->ev[5]));
-    *out = ds;
-    out->off = c->h_off.as<u64>(); out->bytes = c->h_out.as<u8>(); out->on_device = 0;
+    if (c->profiling) TRY(ev_elapsed(c, &c->tm.d2h_ms, EV_D2H0, EV_D2H1));
     return NUTSB_OK;
 }
 
-// Brings a gather-list result to the host (pool, lists) after run_write(..., &iv); ev[4] was recorded before.
+// Gather lists on the host after run_write(..., &iv): as run_write brought them over (plain listeners only),
+// or, for recipients behind filters, one piece per user's stream.
 static int fetch_iov(nutsb_ctx *c, const nutsb_streams &ds, const IovReq &iv, nutsb_iov_streams *out)
 {
-    cudaStream_t st = c->stream;
     const size_t U = (size_t)c->U;
-    u64 n_iov = 0;
     out->pool2 = nullptr; out->pool2_bytes = 0;
     if (iv.compact) {
-        // run_write has brought everything over already (the slab while the planning went on)
-        n_iov = iv.n_iov;
-        out->pool_bytes = iv.slab_span;
+        out->n_iov = iv.n_iov; out->pool_bytes = iv.slab_span;
         out->pool2 = c->h_dir.as<u8>(); out->pool2_bytes = iv.direct_bytes;
     } else {
-        // recipients behind filters (or nothing to send): the streams themselves, one piece per user
-        n_iov = U; out->pool_bytes = ds.total_bytes;
-        TRY(ensure_host(c, c->h_off, (U + 1) * 8));
+        TRY(streams_to_host(c, ds));
         TRY(ensure_host(c, c->h_iov_first, (U + 1) * 8)); TRY(ensure_host(c, c->h_iov_cnt, (U + 1) * 4));
-        TRY(ensure_host(c, c->h_out, (size_t)ds.total_bytes + 16));
         TRY(ensure_host(c, c->h_iov, (U + 1) * sizeof(nutsb_iovec)));
-        CK(cudaMemcpyAsync(c->h_off.p, ds.off, (U + 1) * 8, cudaMemcpyDeviceToHost, st));
-        if (ds.total_bytes) CK(cudaMemcpyAsync(c->h_out.p, ds.bytes, (size_t)ds.total_bytes, cudaMemcpyDeviceToHost, st));
-        if (c->profiling) CK(cudaEventRecord(c->ev[5], st));
-        CK(cudaStreamSynchronize(st));
-        if (c->profiling) CK(cudaEventElapsedTime(&c->tm.d2h_ms, c->ev[4], c->ev[5]));
         const u64 *off = c->h_off.as<u64>();
         nutsb_iovec *v = c->h_iov.as<nutsb_iovec>();
         for (size_t u = 0; u < U; ++u) {
             v[u].base = c->h_out.as<u8>() + off[u]; v[u].len = (size_t)(off[u + 1] - off[u]);
             c->h_iov_first.as<u64>()[u] = u; c->h_iov_cnt.as<u32>()[u] = 1;
         }
+        out->n_iov = U; out->pool_bytes = ds.total_bytes;
     }
     out->n_users = (int64_t)U; out->total_bytes = ds.total_bytes; out->n_deliveries = ds.n_deliveries;
     out->off = c->h_off.as<u64>(); out->first = c->h_iov_first.as<u64>(); out->count = c->h_iov_cnt.as<u32>();
-    out->iov = c->h_iov.as<nutsb_iovec>(); out->n_iov = n_iov;
+    out->iov = c->h_iov.as<nutsb_iovec>();
     out->pool = c->h_out.as<u8>();
     return NUTSB_OK;
 }
 
-// Gather lists (include/nutsb200.h): with plain listeners only, what crosses PCIe is the slab's two
-// renderings, the direct ops' renderings and 16 bytes per piece -- not one copy of the bytes per recipient.
-static int write_batch_iov_host(nutsb_ctx *c, const nutsb_ops *o, nutsb_iov_streams *out)
+// The form a write entry point hands its result over in: streams left in HBM, streams in pinned host memory, or
+// gather lists (include/nutsb200.h: with plain listeners only, what crosses PCIe is the slab's two renderings,
+// the direct ops' renderings and 16 bytes per piece -- not one copy of the bytes per recipient).
+struct Result { enum Form { HBM, HOST, IOV } form; nutsb_streams *st; nutsb_iov_streams *iov; };
+
+// The last step of every write entry point: run_write's result in the requested form, and the copy timings
+// (0 for copies the call did not make).
+static int deliver(nutsb_ctx *c, bool uploaded, const nutsb_streams &ds, const IovReq &iv, const Result &r)
 {
-    if (!out) return fail(c, NUTSB_E_INVAL, "null argument%s");
-    nutsb_streams probe{};
-    TRY(check_ops(c, o, &probe));
-    CK(cudaSetDevice(c->device));
-    cudaStream_t st = c->stream;
-    if (c->profiling) CK(cudaEventRecord(c->ev[4], st));
-    nutsb_ops d;
-    TRY(upload_ops(c, o, &d));
-    if (c->profiling) CK(cudaEventRecord(c->ev[5], st));
-    nutsb_streams ds{}; IovReq iv;
-    TRY(run_write(c, &d, &ds, &iv));
-    if (c->profiling) { CK(cudaEventElapsedTime(&c->tm.h2d_ms, c->ev[4], c->ev[5])); CK(cudaEventRecord(c->ev[4], st)); }
-    return fetch_iov(c, ds, iv, out);
+    if (c->profiling) {
+        c->tm.h2d_ms = 0;
+        if (uploaded) TRY(ev_elapsed(c, &c->tm.h2d_ms, EV_H2D0, EV_H2D1));
+    }
+    if (r.form == Result::IOV) return fetch_iov(c, ds, iv, r.iov);
+    if (r.form == Result::HBM) { if (c->profiling) c->tm.d2h_ms = 0; *r.st = ds; return NUTSB_OK; }
+    TRY(streams_to_host(c, ds));
+    *r.st = ds;
+    r.st->off = c->h_off.as<u64>(); r.st->bytes = c->h_out.as<u8>(); r.st->on_device = 0;
+    return NUTSB_OK;
 }
+
+// A write batch of ops, in HBM or (upload) in host memory.  expanded: the ops have been through the queue's
+// clone / remote expansion.
+static int write_ops(nutsb_ctx *c, const nutsb_ops *o, bool upload, bool expanded, const Result &r)
+{
+    if (!r.st && !r.iov) return fail(c, NUTSB_E_INVAL, "null argument%s");
+    TRY(check_ops(c, o));
+    TRY(begin_write(c, expanded));
+    nutsb_ops d = *o;
+    if (upload) TRY(upload_ops(c, o, &d));
+    nutsb_streams ds{}; IovReq iv;
+    TRY(run_write(c, &d, &ds, r.form == Result::IOV ? &iv : nullptr));
+    return deliver(c, upload, ds, iv, r);
+}
+
+NUTSB_API int nutsb_write_batch_dev(nutsb_ctx *c, const nutsb_ops *o, nutsb_streams *out)
+{ return write_ops(c, o, false, false, { Result::HBM, out, nullptr }); }
+
+// ops in host memory, streams left in HBM (digests, or a later copy, are the caller's business)
+NUTSB_API int nutsb_write_batch_keep(nutsb_ctx *c, const nutsb_ops *o, nutsb_streams *out)
+{ return write_ops(c, o, true, false, { Result::HBM, out, nullptr }); }
 
 static int stream_digests(nutsb_ctx *c, uint64_t *digest, bool cont)
 {
@@ -1290,22 +1371,6 @@ NUTSB_API int nutsb_delivery_digests(nutsb_ctx *c, uint64_t *per_user, uint64_t 
     if (per_user && U) CK(cudaMemcpyAsync(per_user, A.per_user, U * 8, cudaMemcpyDeviceToHost, st));
     if (per_op && n) CK(cudaMemcpyAsync(per_op, A.per_op, (size_t)n * 8, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
-    return NUTSB_OK;
-}
-
-// ops in host memory, streams left in HBM (digests, or a later copy, are the caller's business)
-NUTSB_API int nutsb_write_batch_keep(nutsb_ctx *c, const nutsb_ops *o, nutsb_streams *out)
-{
-    TRY(check_ops(c, o, out));
-    TRY(no_relays_on_device(c));
-    CK(cudaSetDevice(c->device));
-    cudaStream_t st = c->stream;
-    if (c->profiling) CK(cudaEventRecord(c->ev[4], st));
-    nutsb_ops d;
-    TRY(upload_ops(c, o, &d));
-    if (c->profiling) CK(cudaEventRecord(c->ev[5], st));
-    TRY(run_write(c, &d, out));
-    if (c->profiling) { CK(cudaEventElapsedTime(&c->tm.h2d_ms, c->ev[4], c->ev[5])); c->tm.d2h_ms = 0; }
     return NUTSB_OK;
 }
 
@@ -1434,10 +1499,7 @@ NUTSB_API int nutsb_user_banned(nutsb_ctx *c, const char *s) { return verdict_on
 static int q_push_one(nutsb_ctx *c, u8 kind, i32 target, const char *str, size_t n, i32 except_user, u8 flags, i32 gate)
 {
     if (n > NUTSB_MAX_TEXT) return fail(c, NUTSB_E_RANGE, "string longer than NUTSB_MAX_TEXT (2000) bytes%s");
-    c->q_text.insert(c->q_text.end(), (const u8 *)str, (const u8 *)str + n);   // copied: callers reuse text[] at once
-    c->q_off.push_back((u64)c->q_text.size());
-    c->q_kind.push_back(kind); c->q_target.push_back(target); c->q_except.push_back(except_user); c->q_flags.push_back(flags);
-    c->q_gate.push_back(gate);
+    c->q.push(kind, target, (const u8 *)str, n, except_user, flags, gate);     // copied: callers reuse text[] at once
     return NUTSB_OK;
 }
 
@@ -1479,15 +1541,6 @@ static int q_push_user(nutsb_ctx *c, i32 u, const char *str, size_t n, u8 flags,
 //  * every remote user that would have been a recipient of a room / level op gets its frame (q_push_user).
 // All of them at their place in the user list: before the op itself when a clone precedes its (local) owner
 // there, after it otherwise, in list order -- and under the op's own gate.
-struct QMark { size_t text, off, kind, target, except, flags, gate; };
-static QMark q_mark(const nutsb_ctx *c)
-{ return { c->q_text.size(), c->q_off.size(), c->q_kind.size(), c->q_target.size(), c->q_except.size(), c->q_flags.size(), c->q_gate.size() }; }
-static void q_rollback(nutsb_ctx *c, const QMark &m)
-{
-    c->q_text.resize(m.text); c->q_off.resize(m.off); c->q_kind.resize(m.kind); c->q_target.resize(m.target);
-    c->q_except.resize(m.except); c->q_flags.resize(m.flags); c->q_gate.resize(m.gate);
-}
-
 // users flagged as clones / remote users need nutsb_set_clones / nutsb_set_remotes before anything is queued:
 // without them their relays and frames would silently be missing
 static int relays_ready(nutsb_ctx *c)
@@ -1504,9 +1557,9 @@ static int q_push_n(nutsb_ctx *c, u8 kind, i32 target, const char *str, size_t n
 {
     if (!c || !str) return NUTSB_E_INVAL;
     if (c->has_clones) TRY(relays_ready(c));
-    const QMark m = q_mark(c);
+    const HostOps::Mark m = c->q.mark();
     const int rc = q_push_impl(c, kind, target, str, n, except_user, flags, gate);
-    if (rc != NUTSB_OK) q_rollback(c, m);
+    if (rc != NUTSB_OK) c->q.rollback(m);
     return rc;
 }
 static int q_push(nutsb_ctx *c, u8 kind, i32 target, const char *str, i32 except_user, u8 flags, i32 gate = -1)
@@ -1576,8 +1629,8 @@ static int q_push_impl(nutsb_ctx *c, u8 kind, i32 target, const char *str, size_
 
 // Clones (nuts333.h:58-62, 79): owner[u] = index of the clone's owner, -1 for everybody else (a clone is a
 // user flagged NUTSB_UF_CLONE in nutsb_set_users); hear[u] = clone_hear (0 nothing, 1 swears, 2 all).
-// Call after nutsb_set_users.  The relay is made by the queue tier; the batch tier takes ops as they are
-// given (clones simply receive nothing there).
+// Call after nutsb_set_users.  The relay is made by the queue tier's expansion, which the host-buffer batch
+// calls use too; the other write calls refuse the population (begin_write).
 NUTSB_API int nutsb_set_clones(nutsb_ctx *c, int32_t n_users, const int32_t *owner, const uint8_t *hear)
 {
     if (!c || (n_users && (!owner || !hear))) return NUTSB_E_INVAL;
@@ -1639,9 +1692,9 @@ NUTSB_API int nutsb_q_write_level(nutsb_ctx *c, int level, int above, const char
 NUTSB_API int nutsb_q_write_sock(nutsb_ctx *c, int32_t sock_user, const char *str)
 {
     if (!c || !str) return NUTSB_E_INVAL;
-    const QMark m = q_mark(c);
+    const HostOps::Mark m = c->q.mark();
     const int rc = q_push_one(c, NUTSB_OP_USER, sock_user, str, strlen(str), -1, NUTSB_OF_RAW, -1);
-    if (rc != NUTSB_OK) q_rollback(c, m);
+    if (rc != NUTSB_OK) c->q.rollback(m);
     return rc;
 }
 NUTSB_API int nutsb_q_page_line(nutsb_ctx *c, int32_t sock_user, const char *str, int plain)
@@ -1687,7 +1740,7 @@ NUTSB_API int nutsb_q_more(nutsb_ctx *c, int32_t user, int32_t sock_user, const 
     return NUTSB_OK;
 }
 
-NUTSB_API int64_t nutsb_q_pending(const nutsb_ctx *c) { return c ? (int64_t)c->q_kind.size() : 0; }
+NUTSB_API int64_t nutsb_q_pending(const nutsb_ctx *c) { return c ? (int64_t)c->q.n() : 0; }
 
 // record(), nuts333.c:2062-2071: strncpy pads with NULs, byte REVIEW_LEN becomes '\n', the next one NUL.
 static void do_record(nutsb_ctx *c, i32 room, const char *str)
@@ -1765,72 +1818,58 @@ NUTSB_API int nutsb_q_review(nutsb_ctx *c, int32_t user, int32_t room, const cha
 
 static void q_clear(nutsb_ctx *c)
 {
-    c->q_text.clear(); c->q_off.assign(1, 0); c->q_kind.clear(); c->q_target.clear(); c->q_except.clear(); c->q_flags.clear();
-    c->q_gate.clear(); c->q_sw_text.clear(); c->q_sw_off.assign(1, 0); c->q_sw_verdict.clear(); c->q_rec.clear();
+    c->q.clear(); c->q_sw_text.clear(); c->q_sw_off.assign(1, 0); c->q_sw_verdict.clear(); c->q_rec.clear();
 }
 
 // Policy (include/nutsb200.h): the queue is emptied when the batch has run, or when it can never run (a
 // validation error: the same ops would fail again).  After NUTSB_E_NOMEM / NUTSB_E_CUDA the queue -- ops,
 // swear bodies, pending record() calls -- is kept as it was, so that the flush can be tried again; the review
 // buffers take the pending lines only once the batch that delivers them has succeeded.
-static int flush_impl(nutsb_ctx *c, nutsb_streams *out, nutsb_iov_streams *out_iov)
+static int flush_impl(nutsb_ctx *c, const Result &r)
 {
-    if (!c || (!out && !out_iov)) return NUTSB_E_INVAL;
-    nutsb_ops o{};
-    o.n_ops = (i64)c->q_kind.size();
-    static const u8 zero = 0;
-    o.text = c->q_text.empty() ? &zero : c->q_text.data(); o.text_off = c->q_off.data();
-    o.kind = c->q_kind.data(); o.target = c->q_target.data(); o.except_user = c->q_except.data(); o.flags = c->q_flags.data();
+    if (!c || (!r.st && !r.iov)) return NUTSB_E_INVAL;
     // the swear verdicts the queued say/shout/emote lines branch on: one device batch (unless a review took them)
     int rc = resolve_verdicts(c);
     const i64 n_sw = (i64)c->q_sw_off.size() - 1;
-    if (rc == NUTSB_OK && n_sw > 0) { o.gate = c->q_gate.data(); o.verdict = c->q_sw_verdict.data(); }
-    if (rc == NUTSB_OK) rc = out ? write_batch_host(c, &o, out) : write_batch_iov_host(c, &o, out_iov);
+    const nutsb_ops o = c->q.view(rc == NUTSB_OK && n_sw > 0 ? c->q_sw_verdict.data() : nullptr);
+    if (rc == NUTSB_OK) rc = write_ops(c, &o, true, true, r);
     if (rc == NUTSB_OK) rc = resolve_records(c);
     if (rc != NUTSB_E_NOMEM && rc != NUTSB_E_CUDA) q_clear(c);
     return rc;
 }
-NUTSB_API int nutsb_flush(nutsb_ctx *c, nutsb_streams *out) { return flush_impl(c, out, nullptr); }
+NUTSB_API int nutsb_flush(nutsb_ctx *c, nutsb_streams *out) { return flush_impl(c, { Result::HOST, out, nullptr }); }
+NUTSB_API int nutsb_flush_iov(nutsb_ctx *c, nutsb_iov_streams *out) { return flush_impl(c, { Result::IOV, nullptr, out }); }
 
 // The host-buffer batch tier.  With clones / remote users in the population every op goes through the
 // queue tier's expansion (the relays of c:1416-1426, the frames of c:1299-1307, each under the op's own gate)
 // before the batch runs, so that the streams are the reference's here too.
-static int write_batch_public(nutsb_ctx *c, const nutsb_ops *o, nutsb_streams *out, nutsb_iov_streams *out_iov)
+static int write_batch_public(nutsb_ctx *c, const nutsb_ops *o, const Result &r)
 {
-    if (!c || !c->has_clones) return out ? write_batch_host(c, o, out) : write_batch_iov_host(c, o, out_iov);
-    nutsb_streams probe{};
-    TRY(check_ops(c, o, &probe));
+    if (!c || !c->has_clones) return write_ops(c, o, true, false, r);
+    TRY(check_ops(c, o));
     if (!c->have_users) return fail(c, NUTSB_E_STATE, "nutsb_set_users has not been called%s");
-    if (!c->q_kind.empty() || !c->q_rec.empty()) return fail(c, NUTSB_E_STATE, "a batch over a population with clones / remote users needs an empty queue: flush first%s");
+    if (c->q.n() || !c->q_rec.empty()) return fail(c, NUTSB_E_STATE, "a batch over a population with clones / remote users needs an empty queue: flush first%s");
+    const bool gated = o->gate && o->verdict;
     int rc = NUTSB_OK;
     for (i64 i = 0; i < o->n_ops && rc == NUTSB_OK; ++i) {
-        if (o->text_off[i + 1] < o->text_off[i]) { rc = fail(c, NUTSB_E_INVAL, "text_off is not monotone%s"); break; }
-        const u8 k = o->kind[i];
-        if (k == NUTSB_OP_NONE) continue;
-        if (k > NUTSB_OP_LEVEL) { rc = fail(c, NUTSB_E_INVAL, "unknown op kind%s"); break; }
-        const i32 t = o->target[i], x = o->except_user[i];
-        if (x >= c->U || x < -1 || (k == NUTSB_OP_USER && t >= c->U) || (k == NUTSB_OP_ROOM && (t >= c->R || t < -1))) { rc = fail(c, NUTSB_E_RANGE, "user/room index out of range%s"); break; }
+        const char *why = "";
+        if ((rc = host_op_error(o, i, c->U, c->R, &why)) != NUTSB_OK) { rc = fail(c, rc, "%s", why); break; }
+        if (o->kind[i] == NUTSB_OP_NONE) continue;
         static const char none = 0;
         const size_t n = (size_t)(o->text_off[i + 1] - o->text_off[i]);
-        rc = q_push_n(c, k, t, n ? (const char *)o->text + o->text_off[i] : &none, n, x, o->flags[i], o->gate && o->verdict ? o->gate[i] : -1);
+        rc = q_push_n(c, o->kind[i], o->target[i], n ? (const char *)o->text + o->text_off[i] : &none, n, o->except_user[i], o->flags[i], gated ? o->gate[i] : -1);
     }
     if (rc == NUTSB_OK) {
-        nutsb_ops e{};
-        e.n_ops = (i64)c->q_kind.size();
-        static const u8 zero = 0;
-        e.text = c->q_text.empty() ? &zero : c->q_text.data(); e.text_off = c->q_off.data();
-        e.kind = c->q_kind.data(); e.target = c->q_target.data(); e.except_user = c->q_except.data(); e.flags = c->q_flags.data();
-        if (o->gate && o->verdict) { e.gate = c->q_gate.data(); e.verdict = o->verdict; }
-        rc = out ? write_batch_host(c, &e, out) : write_batch_iov_host(c, &e, out_iov);
+        const nutsb_ops e = c->q.view(gated ? o->verdict : nullptr);
+        rc = write_ops(c, &e, true, true, r);
     }
     q_clear(c);
     return rc;
 }
 NUTSB_API int nutsb_write_batch(nutsb_ctx *c, const nutsb_ops *o, nutsb_streams *out)
-{ if (!out) return fail(c, NUTSB_E_INVAL, "null argument%s"); return write_batch_public(c, o, out, nullptr); }
+{ if (!out) return fail(c, NUTSB_E_INVAL, "null argument%s"); return write_batch_public(c, o, { Result::HOST, out, nullptr }); }
 NUTSB_API int nutsb_write_batch_iov(nutsb_ctx *c, const nutsb_ops *o, nutsb_iov_streams *out)
-{ if (!out) return fail(c, NUTSB_E_INVAL, "null argument%s"); return write_batch_public(c, o, nullptr, out); }
-NUTSB_API int nutsb_flush_iov(nutsb_ctx *c, nutsb_iov_streams *out) { return flush_impl(c, nullptr, out); }
+{ if (!out) return fail(c, NUTSB_E_INVAL, "null argument%s"); return write_batch_public(c, o, { Result::IOV, nullptr, out }); }
 
 // ---------------------------------------------------------------------------------------
 // the callers' composition
@@ -1951,7 +1990,7 @@ NUTSB_API int nutsb_q_wizshout(nutsb_ctx *c, int32_t user, int lev, const char *
     if (user < 0 || user >= c->U) return fail(c, NUTSB_E_RANGE, "user index out of range%s");
     if (c->sflags[(size_t)user] & NUTSB_SF_MUZZLED) return nutsb_q_write_user(c, user, "You are muzzled, you cannot wizshout.\n");
     const size_t n_all = strlen(inpstr);
-    const QMark m = q_mark(c);
+    const HostOps::Mark m = c->q.mark();
     const size_t sw_text = c->q_sw_text.size(), sw_off = c->q_sw_off.size();
     i32 gate = -1;
     int rc = NUTSB_OK;
@@ -1972,7 +2011,7 @@ NUTSB_API int nutsb_q_wizshout(nutsb_ctx *c, int32_t user, int lev, const char *
     const std::string b = "~OL" + user_name(c, user) + " wizshouts" + to + ":~RS " + msg + "\n";
     if (rc == NUTSB_OK) rc = q_push(c, NUTSB_OP_USER, user, a.c_str(), -1, 0, gate);
     if (rc == NUTSB_OK) rc = q_push(c, NUTSB_OP_LEVEL, lev >= 0 ? lev : 2 /* WIZ */, b.c_str(), user, NUTSB_OF_ABOVE, gate);
-    if (rc != NUTSB_OK) { q_rollback(c, m); c->q_sw_text.resize(sw_text); c->q_sw_off.resize(sw_off); }
+    if (rc != NUTSB_OK) { c->q.rollback(m); c->q_sw_text.resize(sw_text); c->q_sw_off.resize(sw_off); }
     return rc;
 }
 
@@ -1994,7 +2033,7 @@ NUTSB_API int nutsb_q_revtell(nutsb_ctx *c, int32_t user)
 }
 
 static int run_speech(nutsb_ctx *c, i64 n, const u8 *verb, const i32 *speaker, const u8 *bodies, const u64 *body_off, nutsb_streams *out,
-                      IovReq *iv = nullptr)
+                      IovReq *iv)
 {
     TRY(speech_ready(c));
     cudaStream_t st = c->stream;
@@ -2024,66 +2063,48 @@ static int run_speech(nutsb_ctx *c, i64 n, const u8 *verb, const i32 *speaker, c
     return run_write(c, &o, out, iv);
 }
 
-NUTSB_API int nutsb_speech_batch_dev(nutsb_ctx *c, int64_t n, const uint8_t *verb, const int32_t *speaker,
-                                     const uint8_t *bodies, const uint64_t *body_off, nutsb_streams *out)
+// the n input lines of a speech batch, host memory -> staging buffers in HBM (the pointers are replaced by theirs)
+static int upload_speech(nutsb_ctx *c, i64 n, const u8 *&verb, const i32 *&speaker, const u8 *&bodies, const u64 *&body_off)
 {
-    if (!c || !out || n < 0 || (n && (!verb || !speaker || !body_off))) return fail(c, NUTSB_E_INVAL, "bad argument%s");
-    CK(cudaSetDevice(c->device));
-    return run_speech(c, n, verb, speaker, bodies, body_off, out);
-}
-
-// the n input lines of a speech batch, host memory -> staging buffers in HBM
-static int upload_speech(nutsb_ctx *c, i64 n, const u8 *verb, const i32 *speaker, const u8 *bodies, const u64 *body_off,
-                         const u8 **dv, const i32 **ds, const u8 **db, const u64 **dbo)
-{
-    *dv = nullptr; *ds = nullptr; *db = nullptr; *dbo = nullptr;
-    if (n <= 0) return NUTSB_OK;
+    cudaStream_t st = c->stream;
+    TRY(ev_record(c, EV_H2D0, st));
+    if (n <= 0) return ev_record(c, EV_H2D1, st);
     const u64 t0 = body_off[0], t1 = body_off[n];
     if (t1 < t0 || (t1 > t0 && !bodies)) return fail(c, NUTSB_E_INVAL, "bad body offsets%s");
     // (offsets that are not monotone inside [t0, t1] are caught on the device: k_speech_measure)
     TRY(ensure(c, c->s_body, (size_t)(t1 - t0) + 64));
-    if (t1 > t0) CK(cudaMemcpyAsync(c->s_body.p, bodies + t0, (size_t)(t1 - t0), cudaMemcpyHostToDevice, c->stream));
+    if (t1 > t0) CK(cudaMemcpyAsync(c->s_body.p, bodies + t0, (size_t)(t1 - t0), cudaMemcpyHostToDevice, st));
     TRY(upload(c, c->s_boff, body_off, ((size_t)n + 1) * 8));
     TRY(upload(c, c->s_verb, verb, (size_t)n));
     TRY(upload(c, c->s_speaker, speaker, (size_t)n * 4));
-    *dv = c->s_verb.as<u8>(); *ds = c->s_speaker.as<i32>(); *db = c->s_body.as<u8>() - t0; *dbo = c->s_boff.as<u64>();
-    return NUTSB_OK;
+    verb = c->s_verb.as<u8>(); speaker = c->s_speaker.as<i32>(); bodies = c->s_body.as<u8>() - t0; body_off = c->s_boff.as<u64>();
+    return ev_record(c, EV_H2D1, st);
 }
+
+// A speech batch: the input lines in HBM or (upload) in host memory, composed on the device
+static int speech_batch(nutsb_ctx *c, i64 n, const u8 *verb, const i32 *speaker, const u8 *bodies, const u64 *body_off,
+                        bool upload, const Result &r)
+{
+    if (!c || (!r.st && !r.iov) || n < 0 || (n && (!verb || !speaker || !body_off))) return fail(c, NUTSB_E_INVAL, "bad argument%s");
+    TRY(begin_write(c, false));
+    if (upload) TRY(upload_speech(c, n, verb, speaker, bodies, body_off));
+    nutsb_streams ds{}; IovReq iv;
+    TRY(run_speech(c, n, verb, speaker, bodies, body_off, &ds, r.form == Result::IOV ? &iv : nullptr));
+    return deliver(c, upload, ds, iv, r);
+}
+
+NUTSB_API int nutsb_speech_batch_dev(nutsb_ctx *c, int64_t n, const uint8_t *verb, const int32_t *speaker,
+                                     const uint8_t *bodies, const uint64_t *body_off, nutsb_streams *out)
+{ return speech_batch(c, n, verb, speaker, bodies, body_off, false, { Result::HBM, out, nullptr }); }
 
 NUTSB_API int nutsb_speech_batch(nutsb_ctx *c, int64_t n, const uint8_t *verb, const int32_t *speaker,
                                  const uint8_t *bodies, const uint64_t *body_off, nutsb_streams *out)
-{
-    if (!c || !out || n < 0 || (n && (!verb || !speaker || !body_off))) return fail(c, NUTSB_E_INVAL, "bad argument%s");
-    CK(cudaSetDevice(c->device));
-    const u8 *dv; const i32 *ds; const u8 *db; const u64 *dbo;
-    TRY(upload_speech(c, n, verb, speaker, bodies, body_off, &dv, &ds, &db, &dbo));
-    nutsb_streams ds_{};
-    TRY(run_speech(c, n, dv, ds, db, dbo, &ds_));
-    TRY(ensure_host(c, c->h_off, ((size_t)c->U + 1) * 8));
-    TRY(ensure_host(c, c->h_out, (size_t)ds_.total_bytes + 16));
-    CK(cudaMemcpyAsync(c->h_off.p, ds_.off, ((size_t)c->U + 1) * 8, cudaMemcpyDeviceToHost, c->stream));
-    if (ds_.total_bytes) CK(cudaMemcpyAsync(c->h_out.p, ds_.bytes, (size_t)ds_.total_bytes, cudaMemcpyDeviceToHost, c->stream));
-    CK(cudaStreamSynchronize(c->stream));
-    *out = ds_;
-    out->off = c->h_off.as<u64>(); out->bytes = c->h_out.as<u8>(); out->on_device = 0;
-    return NUTSB_OK;
-}
+{ return speech_batch(c, n, verb, speaker, bodies, body_off, true, { Result::HOST, out, nullptr }); }
 
 // input lines in, gather lists out: the smallest host <-> device traffic the path has (bodies + 5 bytes per
 // line one way; each rendering once per colour setting + 16 bytes per piece the other)
 NUTSB_API int nutsb_speech_batch_iov(nutsb_ctx *c, int64_t n, const uint8_t *verb, const int32_t *speaker,
                                      const uint8_t *bodies, const uint64_t *body_off, nutsb_iov_streams *out)
-{
-    if (!c || !out || n < 0 || (n && (!verb || !speaker || !body_off))) return fail(c, NUTSB_E_INVAL, "bad argument%s");
-    CK(cudaSetDevice(c->device));
-    if (c->profiling) CK(cudaEventRecord(c->ev[4], c->stream));
-    const u8 *dv; const i32 *ds; const u8 *db; const u64 *dbo;
-    TRY(upload_speech(c, n, verb, speaker, bodies, body_off, &dv, &ds, &db, &dbo));
-    if (c->profiling) CK(cudaEventRecord(c->ev[5], c->stream));
-    nutsb_streams ds_{}; IovReq iv;
-    TRY(run_speech(c, n, dv, ds, db, dbo, &ds_, &iv));
-    if (c->profiling) { CK(cudaEventElapsedTime(&c->tm.h2d_ms, c->ev[4], c->ev[5])); CK(cudaEventRecord(c->ev[4], c->stream)); }
-    return fetch_iov(c, ds_, iv, out);
-}
+{ return speech_batch(c, n, verb, speaker, bodies, body_off, true, { Result::IOV, nullptr, out }); }
 
 #include "nutsb_multi.cuh"

@@ -33,10 +33,7 @@ struct nutsb_multi {
     std::vector<std::vector<i32>> shard_users;     // global index of each shard's users, in global order
     std::vector<i32> shard_rooms;                  // rooms per shard
     // routed batch, per shard
-    struct Routed {
-        std::vector<u8> text, kind, flags; std::vector<u64> off; std::vector<i32> target, except_user, gate;
-        nutsb_streams out{}; nutsb_timing tm{}; int rc = NUTSB_OK;
-    };
+    struct Routed { HostOps ops; nutsb_streams out{}; nutsb_timing tm{}; int rc = NUTSB_OK; };
     std::vector<Routed> routed;
     // merged result
     std::vector<u64> len; std::vector<const u8 *> ptr;
@@ -169,51 +166,29 @@ static int multi_route(nutsb_multi *m, const nutsb_ops *o)
         return mfail(m, NUTSB_E_INVAL, "ops array is NULL");
     const int S = m->n_shards;
     const bool gated = o->gate && o->verdict;
-    for (auto &r : m->routed) {
-        r.text.clear(); r.kind.clear(); r.flags.clear(); r.off.assign(1, 0); r.target.clear(); r.except_user.clear(); r.gate.clear();
-        r.rc = NUTSB_OK;
-    }
+    for (auto &r : m->routed) { r.ops.clear(); r.rc = NUTSB_OK; }
     auto push = [&](int s, i64 i, i32 target, i32 exc) {
-        nutsb_multi::Routed &r = m->routed[(size_t)s];
-        r.text.insert(r.text.end(), o->text + o->text_off[i], o->text + o->text_off[i + 1]);
-        r.off.push_back((u64)r.text.size());
-        r.kind.push_back(o->kind[i]); r.flags.push_back(o->flags[i]); r.target.push_back(target); r.except_user.push_back(exc);
-        if (gated) r.gate.push_back(o->gate[i]);
+        m->routed[(size_t)s].ops.push(o->kind[i], target, o->text + o->text_off[i], (size_t)(o->text_off[i + 1] - o->text_off[i]),
+                                      exc, o->flags[i], gated ? o->gate[i] : -1);
     };
     for (i64 i = 0; i < o->n_ops; ++i) {
-        if (o->text_off[i + 1] < o->text_off[i]) return mfail(m, NUTSB_E_INVAL, "text_off is not monotone");
+        const char *why = "";
+        if (const int rc = host_op_error(o, i, m->U, m->R, &why)) return mfail(m, rc, why);
         if (o->text_off[i + 1] - o->text_off[i] > NUTSB_MAX_TEXT) return mfail(m, NUTSB_E_RANGE, "string longer than NUTSB_MAX_TEXT (2000) bytes");
         const u8 k = o->kind[i]; const i32 t = o->target[i], x = o->except_user[i];
         if (k == NUTSB_OP_NONE) continue;
-        if (k > NUTSB_OP_LEVEL) return mfail(m, NUTSB_E_INVAL, "unknown op kind");
-        if (x >= m->U || x < -1) return mfail(m, NUTSB_E_RANGE, "user/room index out of range");
         auto local_x = [&](int s) { return (x >= 0 && m->user_shard[(size_t)x] == s) ? m->user_local[(size_t)x] : -1; };
         if (k == NUTSB_OP_USER) {
-            if (t >= m->U) return mfail(m, NUTSB_E_RANGE, "user/room index out of range");
             if (t < 0) continue;                                       // write_user(NULL, ...): c:1298
             push(m->user_shard[(size_t)t], i, m->user_local[(size_t)t], -1);
         } else if (k == NUTSB_OP_ROOM && t >= 0) {
-            if (t >= m->R) return mfail(m, NUTSB_E_RANGE, "user/room index out of range");
             const int s = m->room_shard[(size_t)t];
             push(s, i, m->room_local[(size_t)t], local_x(s));
         } else {                                                       // all rooms (c:1399) / write_level: every shard
-            if (k == NUTSB_OP_ROOM && t < -1) return mfail(m, NUTSB_E_RANGE, "user/room index out of range");
             for (int s = 0; s < S; ++s) push(s, i, t, local_x(s));
         }
     }
     return NUTSB_OK;
-}
-
-static nutsb_ops routed_ops(const nutsb_multi::Routed &r, const nutsb_ops *o)
-{
-    static const u8 zero = 0; static const i32 zi = 0;
-    nutsb_ops e{};
-    e.n_ops = (i64)r.kind.size();
-    e.text = r.text.empty() ? &zero : r.text.data(); e.text_off = r.off.data();
-    e.kind = r.kind.empty() ? &zero : r.kind.data(); e.flags = r.flags.empty() ? &zero : r.flags.data();
-    e.target = r.target.empty() ? &zi : r.target.data(); e.except_user = r.except_user.empty() ? &zi : r.except_user.data();
-    if (o->gate && o->verdict) { e.gate = r.gate.empty() ? &zi : r.gate.data(); e.verdict = o->verdict; }
-    return e;
 }
 
 // The routed ops of one shard, as host arrays owned by the handle (valid until the next batch): for a caller that
@@ -222,7 +197,7 @@ NUTSB_API int nutsb_multi_route(nutsb_multi *m, const nutsb_ops *ops, int shard,
 {
     if (!m || !out || shard < 0 || shard >= m->n_shards) return NUTSB_E_INVAL;
     TRY(multi_route(m, ops));
-    *out = routed_ops(m->routed[(size_t)shard], ops);
+    *out = m->routed[(size_t)shard].ops.view(ops->gate && ops->verdict ? ops->verdict : nullptr);
     return NUTSB_OK;
 }
 
@@ -237,7 +212,7 @@ NUTSB_API int nutsb_multi_write_batch(nutsb_multi *m, const nutsb_ops *ops, nuts
         if (!m->ctx[(size_t)s]) continue;
         th.emplace_back([m, s, ops, keep] {
             nutsb_multi::Routed &r = m->routed[(size_t)s];
-            const nutsb_ops e = routed_ops(r, ops);
+            const nutsb_ops e = r.ops.view(ops->gate && ops->verdict ? ops->verdict : nullptr);
             r.rc = keep ? nutsb_write_batch_keep(m->ctx[(size_t)s], &e, &r.out) : nutsb_write_batch(m->ctx[(size_t)s], &e, &r.out);
             if (r.rc == NUTSB_OK) nutsb_get_timing(m->ctx[(size_t)s], &r.tm);
         });
