@@ -367,7 +367,8 @@ int nutsb_stream_digests_continue(nutsb_ctx *ctx, uint64_t *digest);
  * thread and one device each, no collective; results come back in GLOBAL user order.  Clones / remote users are
  * refused (NUTSB_E_UNSUPPORTED): their relays cross rooms.
  * nutsb_multi_create_rank: one process per GPU (torchrun) -- this process runs shard `shard` only; every process
- * gives the same population and batches, plans and routes identically, and reports its own users' streams. */
+ * gives the same population and batches, plans and routes identically, and reports its own users' streams
+ * (the users of the other shards come back empty). */
 typedef struct nutsb_multi nutsb_multi;
 typedef struct nutsb_mstreams {
     int64_t         n_users;
@@ -396,6 +397,36 @@ int  nutsb_multi_contains_swearing_batch(nutsb_multi *m, int64_t n, const uint8_
 int  nutsb_multi_site_banned_batch(nutsb_multi *m, int64_t n, const uint8_t *bytes, const uint64_t *off, uint8_t *verdict);
 int  nutsb_multi_user_banned_batch(nutsb_multi *m, int64_t n, const uint8_t *bytes, const uint64_t *off, uint8_t *verdict);
 int  nutsb_multi_get_timing(const nutsb_multi *m, int shard, nutsb_timing *out);
+
+/* Gather lists over the shards (see nutsb_write_batch_iov), in GLOBAL user order: user u's stream is
+ *     writev(sock, (const struct iovec *)s.iov[u], s.count[u]);
+ * iov[u] points at u's first piece inside the gather list of u's shard (no byte is copied); pieces point into
+ * that shard's pools (nutsb_multi_shard_iov).  Valid until the next batch on the handle. */
+typedef struct nutsb_miov_streams {
+    int64_t                   n_users;
+    uint64_t                  total_bytes, n_deliveries;   /* over the shards this process runs          */
+    const uint64_t           *len;     /* n_users: length of user u's stream                          */
+    const nutsb_iovec *const *iov;     /* n_users: u's first piece, inside its shard's iov array      */
+    const uint32_t           *count;   /* n_users: u's pieces (0, iov[u] NULL: a shard not run here)  */
+} nutsb_miov_streams;
+int  nutsb_multi_write_batch_iov(nutsb_multi *m, const nutsb_ops *ops, nutsb_miov_streams *out);
+/* the last gather-list batch's result of one shard as nutsb_write_batch_iov gives it (local user order, its pools) */
+int  nutsb_multi_shard_iov(const nutsb_multi *m, int shard, nutsb_iov_streams *out);
+
+/* Speech batches over the shards (see nutsb_speech_batch).  Names and speech flags in GLOBAL user order, before or
+ * after nutsb_multi_set_users; every speaker index is a global one.  Every shard is given the whole batch and picks,
+ * on the device, the lines that produce an op on it, by the same rule the one-context composer uses: the refusal,
+ * the speaker's own copy and the line to the speaker's room go to the speaker's shard; shout / semote / bcast (all rooms) and echo's
+ * write_level(WIZ) go to every shard.  Each shard takes the swear verdicts of the whole batch.  Streams, totals and
+ * errors as for nutsb_multi_write_batch (keep != 0: the streams stay in HBM, nutsb_multi_stream_digests);
+ * NUTSB_E_STATE when the names do not match the population. */
+int  nutsb_multi_set_user_names(nutsb_multi *m, int32_t n_users, const uint8_t *names, const uint64_t *off,
+                                const uint8_t *speech_flags);
+int  nutsb_multi_set_ban_swearing(nutsb_multi *m, int on);
+int  nutsb_multi_speech_batch(nutsb_multi *m, int64_t n, const uint8_t *verb, const int32_t *speaker,
+                              const uint8_t *bodies, const uint64_t *body_off, nutsb_mstreams *out, int keep);
+int  nutsb_multi_speech_batch_iov(nutsb_multi *m, int64_t n, const uint8_t *verb, const int32_t *speaker,
+                                  const uint8_t *bodies, const uint64_t *body_off, nutsb_miov_streams *out);
 
 /* ---- calls in flight on one device -----------------------------------------------------------------
  * A host-buffer call is H2D copy -> kernels -> D2H copy; PCIe is full duplex, so with two calls in flight one call's

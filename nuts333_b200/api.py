@@ -68,6 +68,11 @@ class _MStreams(C.Structure):
                 ("len", C.c_void_p), ("ptr", C.c_void_p), ("on_device", C.c_int32)]
 
 
+class _MIovStreams(C.Structure):
+    _fields_ = [("n_users", C.c_int64), ("total_bytes", C.c_uint64), ("n_deliveries", C.c_uint64),
+                ("len", C.c_void_p), ("iov", C.c_void_p), ("count", C.c_void_p)]
+
+
 class Timing(C.Structure):
     _fields_ = [("plan_ms", C.c_float), ("render_ms", C.c_float), ("fanout_ms", C.c_float), ("direct_ms", C.c_float),
                 ("total_ms", C.c_float), ("h2d_ms", C.c_float), ("d2h_ms", C.c_float),
@@ -93,6 +98,8 @@ EXPORTS = [
     "nutsb_multi_set_swear_words", "nutsb_multi_set_ban_files", "nutsb_multi_set_profiling", "nutsb_multi_set_users", "nutsb_multi_plan",
     "nutsb_multi_route", "nutsb_multi_write_batch", "nutsb_multi_stream_digests", "nutsb_multi_contains_swearing_batch",
     "nutsb_multi_site_banned_batch", "nutsb_multi_user_banned_batch", "nutsb_multi_get_timing",
+    "nutsb_multi_write_batch_iov", "nutsb_multi_shard_iov", "nutsb_multi_set_user_names", "nutsb_multi_set_ban_swearing",
+    "nutsb_multi_speech_batch", "nutsb_multi_speech_batch_iov",
     "nutsb_pipe_create", "nutsb_pipe_destroy", "nutsb_pipe_depth", "nutsb_pipe_ctx", "nutsb_pipe_set_swear_words", "nutsb_pipe_set_users",
     "nutsb_pipe_set_user_names", "nutsb_pipe_set_ban_swearing", "nutsb_pipe_submit_speech_iov", "nutsb_pipe_submit_write_iov", "nutsb_pipe_wait",
 ]
@@ -183,6 +190,12 @@ def bind(lib: C.CDLL) -> C.CDLL:
     for name in ("contains_swearing", "site_banned", "user_banned"):
         getattr(lib, f"nutsb_multi_{name}_batch").argtypes = [vp, C.c_int64, vp, vp, vp]
     lib.nutsb_multi_get_timing.argtypes = [vp, C.c_int, C.POINTER(Timing)]
+    lib.nutsb_multi_write_batch_iov.argtypes = [vp, C.POINTER(_Ops), C.POINTER(_MIovStreams)]
+    lib.nutsb_multi_shard_iov.argtypes = [vp, C.c_int, C.POINTER(_IovStreams)]
+    lib.nutsb_multi_set_user_names.argtypes = [vp, C.c_int32, vp, vp, vp]
+    lib.nutsb_multi_set_ban_swearing.argtypes = [vp, C.c_int]
+    lib.nutsb_multi_speech_batch.argtypes = [vp, C.c_int64, vp, vp, vp, vp, C.POINTER(_MStreams), C.c_int]
+    lib.nutsb_multi_speech_batch_iov.argtypes = [vp, C.c_int64, vp, vp, vp, vp, C.POINTER(_MIovStreams)]
     lib.nutsb_pipe_create.argtypes = [C.POINTER(vp), C.c_int, C.c_int]
     lib.nutsb_pipe_destroy.argtypes = [vp]
     lib.nutsb_pipe_destroy.restype = None
@@ -654,6 +667,31 @@ class Talker:
         return self.ctx._ck(self.ctx.lib.nutsb_user_banned(self.ctx._h, self._s(name)))
 
 
+class MIovStreams:
+    """Per-user gather lists of a nutsb_multi batch in GLOBAL user order (nutsb_miov_streams): user u's pieces lie in
+    the gather list of u's shard.  Valid until the next batch on the MultiContext."""
+
+    def __init__(self, st):
+        U = int(st.n_users)
+        arr = lambda p, t: np.ctypeslib.as_array(C.cast(p, C.POINTER(t)), shape=(max(U, 1),))[:U].copy()
+        self.len, self.iov_addr, self.count = arr(st.len, C.c_uint64), arr(st.iov, C.c_uint64), arr(st.count, C.c_uint32)
+        self.total_bytes, self.n_deliveries = int(st.total_bytes), int(st.n_deliveries)
+
+    @property
+    def n_users(self):
+        return len(self.len)
+
+    def pieces(self, u):
+        """u64[count[u], 2] = (address, length) of u's pieces"""
+        n = int(self.count[u])
+        if not n:
+            return np.zeros((0, 2), np.uint64)
+        return np.ctypeslib.as_array(C.cast(int(self.iov_addr[u]), u64p), shape=(n, 2)).copy()
+
+    def user(self, u) -> bytes:
+        return b"".join(C.string_at(int(a), int(n)) for a, n in self.pieces(u) if n)
+
+
 class MultiContext:
     """nutsb_multi: one population and one batch over several GPUs (include/nutsb200.h).  `devices`: one context per
     entry (the same device may be named twice); or rank=(n_shards, shard, device) for one process per GPU."""
@@ -752,6 +790,54 @@ class MultiContext:
         ln = np.ctypeslib.as_array(C.cast(st.len, u64p), shape=(max(U, 1),))[:U]
         pt = np.ctypeslib.as_array(C.cast(st.ptr, u64p), shape=(max(U, 1),))[:U]
         return [C.string_at(int(pt[u]), int(ln[u])) if ln[u] else b"" for u in range(U)], int(st.total_bytes), int(st.n_deliveries)
+
+    def write_batch_iov(self, ops) -> MIovStreams:
+        """write_batch with gather lists as the result (nutsb_multi_write_batch_iov)."""
+        k = []
+        o = self._ops(ops, k)
+        st = _MIovStreams()
+        self._ck(self.lib.nutsb_multi_write_batch_iov(self._h, C.byref(o), C.byref(st)))
+        return MIovStreams(st)
+
+    def shard_iov(self, shard) -> IovStreams:
+        """The shard's own result of the last gather-list batch (local user order; its pools hold the pieces)."""
+        st = _IovStreams()
+        self._ck(self.lib.nutsb_multi_shard_iov(self._h, shard, C.byref(st)))
+        return Context._host_iov(None, st)
+
+    def set_user_names(self, names, speech_flags):
+        """names: list[bytes] in global user order; speech_flags: SF_INVIS | SF_MUZZLED per user"""
+        data, off = pack([n if isinstance(n, bytes) else n.encode() for n in names])
+        fl = _np(speech_flags, np.uint8)
+        self._ck(self.lib.nutsb_multi_set_user_names(self._h, len(names), _addr(data) if data.size else None, _addr(off), _addr(fl)))
+
+    def set_ban_swearing(self, on: bool):
+        self._ck(self.lib.nutsb_multi_set_ban_swearing(self._h, 1 if on else 0))
+
+    @staticmethod
+    def _lines(verb, speaker, bodies, body_off):
+        a = (_np(verb, np.uint8), _np(speaker, np.int32), _np(bodies, np.uint8), _np(body_off, np.uint64))
+        return a, (len(a[0]), _addr(a[0]), _addr(a[1]), _addr(a[2]) if a[2].size else None, _addr(a[3]))
+
+    def speech_batch(self, verb, speaker, bodies, body_off, keep=False):
+        """say/shout/emote/semote/echo/bcast lines (global speaker indices) composed on every shard
+        -> list[bytes] per user in GLOBAL order (None when keep), total_bytes, n_deliveries"""
+        arrs, args = self._lines(verb, speaker, bodies, body_off)      # (arrs: the inputs stay alive through the call)
+        st = _MStreams()
+        self._ck(self.lib.nutsb_multi_speech_batch(self._h, *args, C.byref(st), 1 if keep else 0))
+        if keep:
+            return None, int(st.total_bytes), int(st.n_deliveries)
+        U = int(st.n_users)
+        ln = np.ctypeslib.as_array(C.cast(st.len, u64p), shape=(max(U, 1),))[:U]
+        pt = np.ctypeslib.as_array(C.cast(st.ptr, u64p), shape=(max(U, 1),))[:U]
+        return [C.string_at(int(pt[u]), int(ln[u])) if ln[u] else b"" for u in range(U)], int(st.total_bytes), int(st.n_deliveries)
+
+    def speech_batch_iov(self, verb, speaker, bodies, body_off) -> MIovStreams:
+        """speech_batch with gather lists as the result (nutsb_multi_speech_batch_iov)."""
+        arrs, args = self._lines(verb, speaker, bodies, body_off)      # (arrs: the inputs stay alive through the call)
+        st = _MIovStreams()
+        self._ck(self.lib.nutsb_multi_speech_batch_iov(self._h, *args, C.byref(st)))
+        return MIovStreams(st)
 
     def stream_digests(self, digest=None):
         """Per-user digests in global order; digest given: the fold continues from it (chunked jobs)."""

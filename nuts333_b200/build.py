@@ -13,7 +13,7 @@ PKG = Path(__file__).resolve().parent
 CSRC = PKG / "csrc"
 LIB = PKG / "_lib" / "libnutsb200.so"
 SOURCES = [CSRC / "nutsb_lib.cu"]
-HEADERS = [CSRC / "nutsb_common.cuh", CSRC / "nutsb_kernels.cuh", CSRC / "nutsb_match.cuh", CSRC / "nutsb_speech.cuh",
+HEADERS = [CSRC / "nutsb_common.cuh", CSRC / "nutsb_kernels.cuh", CSRC / "nutsb_match.cuh", CSRC / "nutsb_speech.cuh", CSRC / "nutsb_multi.cuh",
            PKG.parent / "include" / "nutsb200.h"]
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

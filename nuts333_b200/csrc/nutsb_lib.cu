@@ -154,6 +154,10 @@ struct nutsb_ctx {
     DBuf d_names, d_name_off, d_sflags, d_lit, d_lit_off;
     DBuf d_sp_len, d_sp_off, d_sp_text, d_sp_kind, d_sp_target, d_sp_except, d_sp_flags, d_sp_gate, d_sp_verdict;
     DBuf s_verb, s_speaker, s_body, s_boff;
+    // the shard mode of the speech batch (nutsb_multi): this context is shard `shard`; the global population's tables
+    // (nutsb_multi_set_users / nutsb_multi_set_user_names) and the lines it selects from a batch
+    i32 shard = -1, g_U = 0; bool have_g_names = false;
+    DBuf d_g_user_shard, d_g_user_local, d_g_has_room, d_g_names, d_g_name_off, d_g_sflags, d_sp_keep, d_sp_sel;
 
     // queue tier
     HostOps q;
@@ -224,6 +228,12 @@ static inline u32 bits_for(u64 n) { u32 b = 0; while (b < 32 && (1ull << b) < n)
 struct InU32 { const u32 *p; __device__ u64 operator()(i64 i) const { return p[i]; } };
 struct InU64 { const u64 *p; __device__ u64 operator()(i64 i) const { return p[i]; } };
 struct InI32 { const i32 *p; __device__ u64 operator()(i64 i) const { return (u64)(i64)p[i]; } };
+struct InU8 { const u8 *p; __device__ u64 operator()(i64 i) const { return p[i]; } };
+// compaction: the indices i < n with keep[i] set, in order, into sel[]; their number into sel[n]
+struct OutSel {
+    const u8 *keep; i32 *sel; i64 n;
+    __device__ void operator()(i64 i, u64 ex) const { if (i == n) sel[n] = (i32)ex; else if (keep[i]) sel[ex] = (i32)i; }
+};
 struct OutU64 { u64 *p; __device__ void operator()(i64 i, u64 ex) const { p[i] = ex; } };
 struct InEntryPacked {
     const u8 *info;
@@ -481,7 +491,8 @@ NUTSB_API void nutsb_destroy(nutsb_ctx *c)
         &c->s_text, &c->s_toff, &c->s_kind, &c->s_target, &c->s_except, &c->s_flags, &c->s_gate, &c->s_verdict, &c->s_v8,
         &c->d_names, &c->d_name_off, &c->d_sflags, &c->d_lit, &c->d_lit_off, &c->d_sp_len, &c->d_sp_off, &c->d_sp_text,
         &c->d_sp_kind, &c->d_sp_target, &c->d_sp_except, &c->d_sp_flags, &c->d_sp_gate, &c->d_sp_verdict,
-        &c->s_verb, &c->s_speaker, &c->s_body, &c->s_boff };
+        &c->s_verb, &c->s_speaker, &c->s_body, &c->s_boff,
+        &c->d_g_user_shard, &c->d_g_user_local, &c->d_g_has_room, &c->d_g_names, &c->d_g_name_off, &c->d_g_sflags, &c->d_sp_keep, &c->d_sp_sel };
     for (DBuf *b : all) release(*b);
     release(c->h_small); release(c->h_off); release(c->h_out);
     release(c->h_dir); release(c->h_iov); release(c->h_iov_first); release(c->h_iov_cnt);
@@ -2032,33 +2043,67 @@ NUTSB_API int nutsb_q_revtell(nutsb_ctx *c, int32_t user)
     return nutsb_q_write_user(c, user, "\n~BB~FG*** End ***\n\n");
 }
 
+// shard: the context is one shard of a nutsb_multi, the speakers are global user indices, and only the lines
+// that produce an op on this shard are composed (k_speech_route, then a scan compacts their indices)
 static int run_speech(nutsb_ctx *c, i64 n, const u8 *verb, const i32 *speaker, const u8 *bodies, const u64 *body_off, nutsb_streams *out,
-                      IovReq *iv)
+                      IovReq *iv, bool shard = false)
 {
     TRY(speech_ready(c));
+    if (shard && (!c->have_g_names || c->shard < 0)) return fail(c, NUTSB_E_STATE, "nutsb_multi_set_user_names does not match the population%s");
     cudaStream_t st = c->stream;
     if (n == 0) { nutsb_ops o{}; return run_write(c, &o, out, iv); }
     SpeechView v{ n, verb, speaker, bodies, body_off, c->d_names.as<u8>(), c->d_name_off.as<u64>(), c->d_sflags.as<u8>(),
                   c->d_user_room.as<i32>(), c->d_lit.as<u8>(), c->d_lit_off.as<u32>(), c->U, c->R, c->ban_swearing ? 1u : 0u };
+    SpeechShard sh{};
+    u64 *h64 = c->h_small.as<u64>(); u32 *h32 = c->h_small.as<u32>();
+    i64 k = n;                                                 // the lines composed here
+    if (shard) {
+        v.names = c->d_g_names.as<u8>(); v.name_off = c->d_g_name_off.as<u64>(); v.sflags = c->d_g_sflags.as<u8>(); v.n_users = c->g_U;
+        sh = SpeechShard{ nullptr, 0, c->d_g_user_shard.as<i32>(), c->d_g_user_local.as<i32>(), c->d_g_has_room.as<u8>(), c->shard };
+        TRY(ensure(c, c->d_sp_keep, (size_t)n)); TRY(ensure(c, c->d_sp_sel, ((size_t)n + 1) * 4));
+    }
     const size_t n3 = (size_t)n * 3;
     TRY(ensure(c, c->d_sp_len, n3 * 4)); TRY(ensure(c, c->d_sp_off, (n3 + 1) * 8));
     TRY(ensure(c, c->d_sp_kind, n3)); TRY(ensure(c, c->d_sp_flags, n3));
     TRY(ensure(c, c->d_sp_target, n3 * 4)); TRY(ensure(c, c->d_sp_except, n3 * 4)); TRY(ensure(c, c->d_sp_gate, n3 * 4));
     TRY(ensure(c, c->d_sp_verdict, (size_t)n));
     CK(cudaMemsetAsync(c->d_status.p, 0, 64, st));
-    NUTSB_LAUNCH(cdiv(n, 256), 256, st, k_speech_measure, v, c->d_sp_len.as<u32>(), c->d_status.as<u32>()); CKL();
-    TRY(run_scan(c, InU32{c->d_sp_len.as<u32>()}, OutU64{c->d_sp_off.as<u64>()}, (i64)n3, nullptr));
-    u64 *h64 = c->h_small.as<u64>(); u32 *h32 = c->h_small.as<u32>();
-    CK(cudaMemcpyAsync(h64, c->d_sp_off.as<u64>() + n3, 8, cudaMemcpyDeviceToHost, st));
+    if (shard) {
+        i32 *sel = c->d_sp_sel.as<i32>();
+        NUTSB_LAUNCH(cdiv(n, 256), 256, st, k_speech_route, v, sh, c->d_sp_keep.as<u8>(), c->d_status.as<u32>()); CKL();
+        TRY(run_scan(c, InU8{c->d_sp_keep.as<u8>()}, OutSel{c->d_sp_keep.as<u8>(), sel, n}, n, nullptr));
+        CK(cudaMemcpyAsync(h32, sel + n, 4, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        k = (i64)h32[0]; sh.sel = sel; sh.k = k;
+        if (k == 0) {                                          // nothing lands here (the line checks still count)
+            CK(cudaMemcpyAsync(h32 + 4, c->d_status.p, 4, cudaMemcpyDeviceToHost, st));
+            CK(cudaStreamSynchronize(st));
+            TRY(status_to_error(c, h32[4]));
+            nutsb_ops o{}; return run_write(c, &o, out, iv);
+        }
+    }
+    const size_t k3 = (size_t)k * 3;
+    if (shard) { NUTSB_LAUNCH(cdiv(k, 256), 256, st, k_speech_measure<true>, v, sh, c->d_sp_len.as<u32>(), c->d_status.as<u32>()); }
+    else       { NUTSB_LAUNCH(cdiv(n, 256), 256, st, k_speech_measure<false>, v, sh, c->d_sp_len.as<u32>(), c->d_status.as<u32>()); }
+    CKL();
+    TRY(run_scan(c, InU32{c->d_sp_len.as<u32>()}, OutU64{c->d_sp_off.as<u64>()}, (i64)k3, nullptr));
+    CK(cudaMemcpyAsync(h64, c->d_sp_off.as<u64>() + k3, 8, cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(h32 + 4, c->d_status.p, 4, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     TRY(status_to_error(c, h32[4]));
     const u64 text_bytes = h64[0];
     TRY(ensure(c, c->d_sp_text, text_bytes + 64));
-    NUTSB_LAUNCH(cdiv((u64)n * NUTSB_SPEECH_GROUP, 256), 256, st, k_speech_compose, v, c->d_sp_off.as<u64>(), c->d_sp_text.as<u8>(),
-                 c->d_sp_kind.as<u8>(), c->d_sp_target.as<i32>(), c->d_sp_except.as<i32>(), c->d_sp_flags.as<u8>(), c->d_sp_gate.as<i32>()); CKL();
+    if (shard) {
+        NUTSB_LAUNCH(cdiv((u64)k * NUTSB_SPEECH_GROUP, 256), 256, st, k_speech_compose<true>, v, sh, c->d_sp_off.as<u64>(), c->d_sp_text.as<u8>(),
+                     c->d_sp_kind.as<u8>(), c->d_sp_target.as<i32>(), c->d_sp_except.as<i32>(), c->d_sp_flags.as<u8>(), c->d_sp_gate.as<i32>());
+    } else {
+        NUTSB_LAUNCH(cdiv((u64)n * NUTSB_SPEECH_GROUP, 256), 256, st, k_speech_compose<false>, v, sh, c->d_sp_off.as<u64>(), c->d_sp_text.as<u8>(),
+                     c->d_sp_kind.as<u8>(), c->d_sp_target.as<i32>(), c->d_sp_except.as<i32>(), c->d_sp_flags.as<u8>(), c->d_sp_gate.as<i32>());
+    }
+    CKL();
+    // the verdicts of every line: a shard delivers gated shouts of speakers who live elsewhere (the gates are line indices)
     TRY(verdict_dev(c, V_SWEAR, n, bodies, body_off, c->d_sp_verdict.as<u8>()));
-    nutsb_ops o{ (i64)n3, c->d_sp_text.as<u8>(), c->d_sp_off.as<u64>(), c->d_sp_kind.as<u8>(), c->d_sp_target.as<i32>(),
+    nutsb_ops o{ (i64)k3, c->d_sp_text.as<u8>(), c->d_sp_off.as<u64>(), c->d_sp_kind.as<u8>(), c->d_sp_target.as<i32>(),
                  c->d_sp_except.as<i32>(), c->d_sp_flags.as<u8>(), c->d_sp_gate.as<i32>(), c->d_sp_verdict.as<u8>() };
     return run_write(c, &o, out, iv);
 }
@@ -2083,13 +2128,13 @@ static int upload_speech(nutsb_ctx *c, i64 n, const u8 *&verb, const i32 *&speak
 
 // A speech batch: the input lines in HBM or (upload) in host memory, composed on the device
 static int speech_batch(nutsb_ctx *c, i64 n, const u8 *verb, const i32 *speaker, const u8 *bodies, const u64 *body_off,
-                        bool upload, const Result &r)
+                        bool upload, const Result &r, bool shard = false)
 {
     if (!c || (!r.st && !r.iov) || n < 0 || (n && (!verb || !speaker || !body_off))) return fail(c, NUTSB_E_INVAL, "bad argument%s");
     TRY(begin_write(c, false));
     if (upload) TRY(upload_speech(c, n, verb, speaker, bodies, body_off));
     nutsb_streams ds{}; IovReq iv;
-    TRY(run_speech(c, n, verb, speaker, bodies, body_off, &ds, r.form == Result::IOV ? &iv : nullptr));
+    TRY(run_speech(c, n, verb, speaker, bodies, body_off, &ds, r.form == Result::IOV ? &iv : nullptr, shard));
     return deliver(c, upload, ds, iv, r);
 }
 

@@ -11,7 +11,11 @@
 //     for its own users; user / room indices become the shard's local ones, an excluded user who lives
 //     elsewhere becomes "nobody" (he is in none of this shard's rooms); swear verdicts are replicated;
 //   * every shard runs on its own device, one host thread each, no collective; the results come back in
-//     GLOBAL user order.
+//     GLOBAL user order: streams (nutsb_mstreams) or gather lists (nutsb_miov_streams), by pointer
+//     bookkeeping over the shards' own results;
+//   * a speech batch (nutsb_multi_speech_batch*) is not routed on the host: every shard is given the whole
+//     batch and picks the lines that produce an op on it on the device (k_speech_route), by the rule the one-
+//     context composer uses (nutsb_speech_slot).
 // A shard whose context is absent (nutsb_multi_create_rank: one process per GPU, torchrun) is planned and
 // routed but not run: its users' streams are reported empty by this process.
 #include <thread>
@@ -32,11 +36,15 @@ struct nutsb_multi {
     std::vector<i32> room_shard, room_local, user_shard, user_local;
     std::vector<std::vector<i32>> shard_users;     // global index of each shard's users, in global order
     std::vector<i32> shard_rooms;                  // rooms per shard
-    // routed batch, per shard
-    struct Routed { HostOps ops; nutsb_streams out{}; nutsb_timing tm{}; int rc = NUTSB_OK; };
+    // speech: the global names / speech flags (nutsb_multi_set_user_names), pushed to the shards with the plan
+    bool have_names = false;
+    std::vector<u8> names, sflags; std::vector<u64> name_off;
+    // routed batch and result, per shard
+    struct Routed { HostOps ops; nutsb_streams out{}; nutsb_iov_streams iov{}; nutsb_timing tm{}; int rc = NUTSB_OK; };
     std::vector<Routed> routed;
     // merged result
     std::vector<u64> len; std::vector<const u8 *> ptr;
+    std::vector<const nutsb_iovec *> iov; std::vector<u32> count;
     std::vector<u64> dg_local;
 };
 
@@ -92,6 +100,71 @@ NUTSB_API int nutsb_multi_set_ban_files(nutsb_multi *m, const void *siteban, siz
 NUTSB_API int nutsb_multi_set_profiling(nutsb_multi *m, int on)
 { if (!m) return NUTSB_E_INVAL; MEACH(nutsb_set_profiling(c_, on)); return NUTSB_OK; }
 
+// The speech batch's view of the global population on shard s's device: which shard and local index every user
+// has, and whether the user is in a room.
+static int shard_tables(nutsb_ctx *c, int s, const nutsb_multi *m, const int32_t *room)
+{
+    std::vector<u8> has_room((size_t)m->U);
+    for (i32 u = 0; u < m->U; ++u) has_room[(size_t)u] = room[u] >= 0;
+    c->shard = s; c->g_U = m->U; c->have_g_names = false;
+    TRY(upload(c, c->d_g_user_shard, m->user_shard.data(), (size_t)m->U * 4));
+    TRY(upload(c, c->d_g_user_local, m->user_local.data(), (size_t)m->U * 4));
+    TRY(upload(c, c->d_g_has_room, has_room.data(), (size_t)m->U));
+    CK(cudaStreamSynchronize(c->stream));                      // has_room goes out of scope
+    return NUTSB_OK;
+}
+
+// The names to every shard this process runs: its own users' (nutsb_set_user_names: its queue tier) and the global
+// table (the speech batch's names, which a shard needs for the shouts of speakers who live elsewhere).
+static int multi_push_names(nutsb_multi *m)
+{
+    for (int s = 0; s < m->n_shards; ++s) {
+        nutsb_ctx *c = m->ctx[(size_t)s];
+        if (!c) continue;
+        const std::vector<i32> &us = m->shard_users[(size_t)s];
+        std::vector<u8> ln, lf(us.size()); std::vector<u64> lo(us.size() + 1, 0);
+        for (size_t i = 0; i < us.size(); ++i) {
+            const size_t u = (size_t)us[i];
+            ln.insert(ln.end(), m->names.begin() + (ptrdiff_t)m->name_off[u], m->names.begin() + (ptrdiff_t)m->name_off[u + 1]);
+            lo[i + 1] = ln.size(); lf[i] = m->sflags[u];
+        }
+        static const u8 zb = 0;
+        int rc = nutsb_set_user_names(c, (i32)us.size(), ln.empty() ? &zb : ln.data(), lo.data(), lf.empty() ? &zb : lf.data());
+        if (rc == NUTSB_OK) rc = [&]() -> int {
+            c->have_g_names = false;
+            TRY(upload(c, c->d_g_names, m->names.data(), m->names.size()));
+            TRY(upload(c, c->d_g_name_off, m->name_off.data(), m->name_off.size() * 8));
+            TRY(upload(c, c->d_g_sflags, m->sflags.data(), m->sflags.size()));
+            CK(cudaStreamSynchronize(c->stream));
+            c->have_g_names = true;
+            return NUTSB_OK;
+        }();
+        if (rc != NUTSB_OK) { m->err = nutsb_last_error(c); return rc; }
+    }
+    return NUTSB_OK;
+}
+
+// user->name, user->vis, user->muzzled of every user in GLOBAL order (as nutsb_set_user_names); may come before or
+// after nutsb_multi_set_users, and is given to the shards whenever the plan changes.
+NUTSB_API int nutsb_multi_set_user_names(nutsb_multi *m, int32_t n_users, const uint8_t *names, const uint64_t *off, const uint8_t *sflags)
+{
+    if (!m || n_users < 0 || (n_users && (!off || !sflags))) return mfail(m, NUTSB_E_INVAL, "nutsb_multi_set_user_names: bad argument");
+    if (m->have_users && n_users != m->U) return mfail(m, NUTSB_E_STATE, "nutsb_multi_set_user_names does not match the population");
+    for (i32 u = 0; u < n_users; ++u) if (off[u + 1] < off[u]) return mfail(m, NUTSB_E_INVAL, "name offsets are not monotone");
+    const u64 t0 = n_users ? off[0] : 0, t1 = n_users ? off[n_users] : 0;
+    if (t1 > t0 && !names) return mfail(m, NUTSB_E_INVAL, "names is NULL");
+    m->have_names = false;
+    m->names.assign(names ? names + t0 : nullptr, names ? names + t1 : nullptr);
+    m->name_off.assign((size_t)n_users + 1, 0);
+    for (i32 u = 0; u <= n_users; ++u) m->name_off[(size_t)u] = n_users ? off[u] - t0 : 0;
+    m->sflags.assign(sflags, sflags + n_users);
+    m->have_names = true;
+    return m->have_users ? multi_push_names(m) : NUTSB_OK;
+}
+
+NUTSB_API int nutsb_multi_set_ban_swearing(nutsb_multi *m, int on)
+{ if (!m) return NUTSB_E_INVAL; MEACH(nutsb_set_ban_swearing(c_, on)); return NUTSB_OK; }
+
 // The global population (index = position in the reference's user list).  room_weight: per room, the load it
 // is expected to bring (NULL: its population).
 NUTSB_API int nutsb_multi_set_users(nutsb_multi *m, int32_t n_users, int32_t n_rooms, const int32_t *room,
@@ -140,11 +213,14 @@ NUTSB_API int nutsb_multi_set_users(nutsb_multi *m, int32_t n_users, int32_t n_r
             lr[i] = room[u] >= 0 ? m->room_local[(size_t)room[u]] : -1; lf[i] = flags[u]; ll[i] = level[u];
         }
         static const i32 zi = 0; static const u8 zb = 0;
-        const int rc = nutsb_set_users(c, (i32)us.size(), m->shard_rooms[(size_t)s], us.empty() ? &zi : lr.data(), us.empty() ? &zb : lf.data(), us.empty() ? &zb : ll.data());
+        int rc = nutsb_set_users(c, (i32)us.size(), m->shard_rooms[(size_t)s], us.empty() ? &zi : lr.data(), us.empty() ? &zb : lf.data(), us.empty() ? &zb : ll.data());
+        if (rc == NUTSB_OK) rc = shard_tables(c, s, m, room);
         if (rc != NUTSB_OK) { m->err = nutsb_last_error(c); return rc; }
     }
     m->len.assign((size_t)n_users, 0); m->ptr.assign((size_t)n_users, nullptr);
+    m->iov.assign((size_t)n_users, nullptr); m->count.assign((size_t)n_users, 0);
     m->have_users = true;
+    if (m->have_names && (i32)m->sflags.size() == n_users) return multi_push_names(m);       // the plan moved users between shards
     return NUTSB_OK;
 }
 
@@ -201,19 +277,22 @@ NUTSB_API int nutsb_multi_route(nutsb_multi *m, const nutsb_ops *ops, int shard,
     return NUTSB_OK;
 }
 
-/* keep != 0: the streams stay in HBM (ptr[] NULL); digests through nutsb_multi_stream_digests */
-NUTSB_API int nutsb_multi_write_batch(nutsb_multi *m, const nutsb_ops *ops, nutsb_mstreams *out, int keep)
+// The result forms of a batch over the shards: streams on the host, streams kept in HBM, gather lists.
+enum MForm { M_STREAMS, M_KEEP, M_IOV };
+
+// One batch on every shard this process runs, one host thread each (job: the shard's call, its result into
+// r.out / r.iov), then the merge into global user order -- pointer bookkeeping over the shards' own results, no
+// byte copied.  If a shard fails: its code and message, and the output is left alone.
+template <class Job>
+static int multi_batch(nutsb_multi *m, MForm form, Job job, nutsb_mstreams *ms, nutsb_miov_streams *mi)
 {
-    if (!m || !out) return NUTSB_E_INVAL;
-    TRY(multi_route(m, ops));
     const int S = m->n_shards;
     std::vector<std::thread> th;
     for (int s = 0; s < S; ++s) {
         if (!m->ctx[(size_t)s]) continue;
-        th.emplace_back([m, s, ops, keep] {
+        th.emplace_back([m, s, &job] {
             nutsb_multi::Routed &r = m->routed[(size_t)s];
-            const nutsb_ops e = r.ops.view(ops->gate && ops->verdict ? ops->verdict : nullptr);
-            r.rc = keep ? nutsb_write_batch_keep(m->ctx[(size_t)s], &e, &r.out) : nutsb_write_batch(m->ctx[(size_t)s], &e, &r.out);
+            r.rc = job(m->ctx[(size_t)s], r);
             if (r.rc == NUTSB_OK) nutsb_get_timing(m->ctx[(size_t)s], &r.tm);
         });
         NUTSB_MULTI_SERIAL(th);
@@ -221,22 +300,91 @@ NUTSB_API int nutsb_multi_write_batch(nutsb_multi *m, const nutsb_ops *ops, nuts
     for (auto &t : th) t.join();
     for (int s = 0; s < S; ++s)
         if (m->ctx[(size_t)s] && m->routed[(size_t)s].rc != NUTSB_OK) { m->err = nutsb_last_error(m->ctx[(size_t)s]); return m->routed[(size_t)s].rc; }
-    // merge: global user order
     u64 total = 0, deliv = 0;
     std::fill(m->len.begin(), m->len.end(), 0); std::fill(m->ptr.begin(), m->ptr.end(), nullptr);
+    std::fill(m->iov.begin(), m->iov.end(), nullptr); std::fill(m->count.begin(), m->count.end(), 0);
     for (int s = 0; s < S; ++s) {
         if (!m->ctx[(size_t)s]) continue;
         const nutsb_multi::Routed &r = m->routed[(size_t)s];
-        total += r.out.total_bytes; deliv += r.out.n_deliveries;
-        if (keep) continue;                                            // (lengths come with the digests' companion call below)
+        total += form == M_IOV ? r.iov.total_bytes : r.out.total_bytes;
+        deliv += form == M_IOV ? r.iov.n_deliveries : r.out.n_deliveries;
+        if (form == M_KEEP) continue;                                  // (the streams stay in HBM: nutsb_multi_stream_digests)
+        const u64 *off = form == M_IOV ? r.iov.off : r.out.off;
         const std::vector<i32> &us = m->shard_users[(size_t)s];
         for (size_t i = 0; i < us.size(); ++i) {
-            m->len[(size_t)us[i]] = r.out.off[i + 1] - r.out.off[i];
-            m->ptr[(size_t)us[i]] = r.out.bytes + r.out.off[i];
+            const size_t u = (size_t)us[i];
+            m->len[u] = off[i + 1] - off[i];
+            if (form == M_IOV) { m->iov[u] = r.iov.iov + r.iov.first[i]; m->count[u] = r.iov.count[i]; }
+            else m->ptr[u] = r.out.bytes + off[i];
         }
     }
-    out->n_users = m->U; out->total_bytes = total; out->n_deliveries = deliv;
-    out->len = keep ? nullptr : m->len.data(); out->ptr = keep ? nullptr : m->ptr.data(); out->on_device = keep ? 1 : 0;
+    if (form == M_IOV) {
+        mi->n_users = m->U; mi->total_bytes = total; mi->n_deliveries = deliv;
+        mi->len = m->len.data(); mi->iov = m->iov.data(); mi->count = m->count.data();
+    } else {
+        const bool keep = form == M_KEEP;
+        ms->n_users = m->U; ms->total_bytes = total; ms->n_deliveries = deliv;
+        ms->len = keep ? nullptr : m->len.data(); ms->ptr = keep ? nullptr : m->ptr.data(); ms->on_device = keep ? 1 : 0;
+    }
+    return NUTSB_OK;
+}
+
+// a routed write batch: every shard's share through the one-context call of the form
+static int multi_write(nutsb_multi *m, const nutsb_ops *ops, MForm form, nutsb_mstreams *ms, nutsb_miov_streams *mi)
+{
+    TRY(multi_route(m, ops));
+    const u8 *verdict = ops->gate && ops->verdict ? ops->verdict : nullptr;
+    return multi_batch(m, form, [verdict, form](nutsb_ctx *c, nutsb_multi::Routed &r) {
+        const nutsb_ops e = r.ops.view(verdict);
+        return form == M_IOV ? nutsb_write_batch_iov(c, &e, &r.iov) : form == M_KEEP ? nutsb_write_batch_keep(c, &e, &r.out) : nutsb_write_batch(c, &e, &r.out);
+    }, ms, mi);
+}
+
+/* keep != 0: the streams stay in HBM (ptr[] NULL); digests through nutsb_multi_stream_digests */
+NUTSB_API int nutsb_multi_write_batch(nutsb_multi *m, const nutsb_ops *ops, nutsb_mstreams *out, int keep)
+{
+    if (!m || !out) return NUTSB_E_INVAL;
+    return multi_write(m, ops, keep ? M_KEEP : M_STREAMS, out, nullptr);
+}
+
+NUTSB_API int nutsb_multi_write_batch_iov(nutsb_multi *m, const nutsb_ops *ops, nutsb_miov_streams *out)
+{
+    if (!m || !out) return NUTSB_E_INVAL;
+    return multi_write(m, ops, M_IOV, nullptr, out);
+}
+
+// A speech batch: the whole batch to every shard, which composes the lines that produce an op on it (run_speech's
+// shard mode); speakers are global user indices.
+static int multi_speech(nutsb_multi *m, i64 n, const u8 *verb, const i32 *speaker, const u8 *bodies, const u64 *body_off,
+                        MForm form, nutsb_mstreams *ms, nutsb_miov_streams *mi)
+{
+    if (!m->have_users) return mfail(m, NUTSB_E_STATE, "nutsb_multi_set_users has not been called");
+    if (!m->have_names || (i32)m->sflags.size() != m->U) return mfail(m, NUTSB_E_STATE, "nutsb_multi_set_user_names does not match the population");
+    return multi_batch(m, form, [=](nutsb_ctx *c, nutsb_multi::Routed &r) {
+        const Result res = form == M_IOV ? Result{ Result::IOV, nullptr, &r.iov } : Result{ form == M_KEEP ? Result::HBM : Result::HOST, &r.out, nullptr };
+        return speech_batch(c, n, verb, speaker, bodies, body_off, true, res, true);
+    }, ms, mi);
+}
+
+NUTSB_API int nutsb_multi_speech_batch(nutsb_multi *m, int64_t n, const uint8_t *verb, const int32_t *speaker,
+                                       const uint8_t *bodies, const uint64_t *body_off, nutsb_mstreams *out, int keep)
+{
+    if (!m || !out) return NUTSB_E_INVAL;
+    return multi_speech(m, n, verb, speaker, bodies, body_off, keep ? M_KEEP : M_STREAMS, out, nullptr);
+}
+
+NUTSB_API int nutsb_multi_speech_batch_iov(nutsb_multi *m, int64_t n, const uint8_t *verb, const int32_t *speaker,
+                                           const uint8_t *bodies, const uint64_t *body_off, nutsb_miov_streams *out)
+{
+    if (!m || !out) return NUTSB_E_INVAL;
+    return multi_speech(m, n, verb, speaker, bodies, body_off, M_IOV, nullptr, out);
+}
+
+// One shard's own result of the last gather-list batch (local user order): the pools the merged pieces point into.
+NUTSB_API int nutsb_multi_shard_iov(const nutsb_multi *m, int shard, nutsb_iov_streams *out)
+{
+    if (!m || !out || shard < 0 || shard >= m->n_shards || !m->ctx[(size_t)shard]) return NUTSB_E_INVAL;
+    *out = m->routed[(size_t)shard].iov;
     return NUTSB_OK;
 }
 

@@ -138,6 +138,68 @@ struct SpeechView {
     u32 ban_swearing;
 };
 
+// Shard mode (nutsb_multi): every shard is given the whole batch and composes the lines that produce an op
+// on it.  The speaker index of a line is GLOBAL; the SpeechView's names / name_off / sflags are the global
+// tables, its user_room / n_rooms the shard's own.  Where a slot's op lands: write_user and the speaker's
+// room -> the speaker's shard (a room's users live with it); all rooms (target -1: shout / semote / bcast)
+// and write_level (echo) -> every shard.
+struct SpeechShard {
+    const i32 *sel;          // [k] the lines this shard composes, in batch order (k_speech_route + a scan)
+    i64 k;
+    const i32 *user_shard, *user_local;          // [n_users], global
+    const u8  *has_room;     // [n_users], global: the user is in a room
+    i32 shard;
+};
+
+// The rule's view of speaker `spk` (global) on this shard: on its own shard the local index and room, elsewhere
+// the global index (it only names the speaker's name) and a room that only says whether it has one.
+__device__ __forceinline__ bool nutsb_speech_home(const SpeechView &v, const SpeechShard &sh, i32 spk, i32 *who, i32 *room)
+{
+    const bool home = sh.user_shard[spk] == sh.shard;
+    if (home) {
+        *who = sh.user_local[spk];
+        *room = v.user_room[*who] < v.n_rooms ? v.user_room[*who] : -1;
+    } else {
+        *who = spk; *room = sh.has_room[spk] ? 0 : -1;
+    }
+    return home;
+}
+
+// The slot as this shard delivers it: away from the speaker's shard only the all-room and level ops are left,
+// and nobody is excluded (the speaker is in none of this shard's rooms).
+__device__ __forceinline__ void nutsb_speech_away(SpeechSlot &s)
+{
+    if (s.kind == NUTSB_OP_USER || (s.kind == NUTSB_OP_ROOM && s.target >= 0)) s.kind = NUTSB_OP_NONE;
+    s.except_user = -1;
+}
+
+// One thread per line of the whole batch: keep[m] = line m produces an op on this shard.  The line checks of
+// k_speech_measure are made here, for every line, so that each shard reports what one context would.
+__global__ void __launch_bounds__(256)
+k_speech_route(SpeechView v, SpeechShard sh, u8 *keep, u32 *status)
+{
+    const i64 m = (i64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (m >= v.n) return;
+    keep[m] = 0;
+    const i32 spk = v.speaker[m];
+    const u32 verb = v.verb[m];
+    if (spk < 0 || spk >= v.n_users || verb >= NUTSB_SPEECH_VERBS) {
+        atomicOr(status, spk < 0 || spk >= v.n_users ? NUTSB_ST_BAD_INDEX : NUTSB_ST_BAD_KIND);
+        return;
+    }
+    const u64 b0 = v.body_off[m], b1 = v.body_off[m + 1];
+    if (b1 < b0 || b0 < v.body_off[0] || b1 > v.body_off[v.n]) { atomicOr(status, NUTSB_ST_BAD_OFFSETS); return; }
+    const u8 first = b1 > b0 ? v.body[b0] : 0, last = b1 > b0 ? v.body[b1 - 1] : 0;
+    const bool home = sh.user_shard[spk] == sh.shard;
+    const i32 room = sh.has_room[spk] ? 0 : -1;          // (the rule asks only whether there is one)
+    bool any = false;
+    for (u32 s = 0; s < 3; ++s) {
+        const SpeechSlot sl = nutsb_speech_slot(verb, s, spk, room, v.sflags[spk], v.ban_swearing != 0, first, last);
+        any |= sl.kind != NUTSB_OP_NONE && (home || sl.kind == NUTSB_OP_LEVEL || (sl.kind == NUTSB_OP_ROOM && sl.target < 0));
+    }
+    keep[m] = any ? 1 : 0;
+}
+
 __device__ __forceinline__ u32 nutsb_speech_len(const SpeechView &v, const SpeechSlot &s, i32 spk, u32 blen)
 {
     if (s.kind == NUTSB_OP_NONE) return 0;
@@ -148,33 +210,40 @@ __device__ __forceinline__ u32 nutsb_speech_len(const SpeechView &v, const Speec
     return n;
 }
 
-// One thread per message: the three slot lengths (0 for an unused slot).
+// One thread per message: the three slot lengths (0 for an unused slot).  SHARD: one thread per selected line
+// j (line sel[j]); its slots are ops 3j..3j+2.
+template <bool SHARD>
 __global__ void __launch_bounds__(256)
-k_speech_measure(SpeechView v, u32 *slot_len, u32 *status)
+k_speech_measure(SpeechView v, SpeechShard sh, u32 *slot_len, u32 *status)
 {
-    const i64 m = (i64)blockIdx.x * blockDim.x + threadIdx.x;
-    if (m >= v.n) return;
+    const i64 j = (i64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= (SHARD ? sh.k : v.n)) return;
+    const i64 m = SHARD ? (i64)sh.sel[j] : j;
     const i32 spk = v.speaker[m];
     const u32 verb = v.verb[m];
     if (spk < 0 || spk >= v.n_users || verb >= NUTSB_SPEECH_VERBS) {
         atomicOr(status, spk < 0 || spk >= v.n_users ? NUTSB_ST_BAD_INDEX : NUTSB_ST_BAD_KIND);
-        slot_len[3 * m] = slot_len[3 * m + 1] = slot_len[3 * m + 2] = 0;
+        slot_len[3 * j] = slot_len[3 * j + 1] = slot_len[3 * j + 2] = 0;
         return;
     }
     const u64 b0 = v.body_off[m], b1 = v.body_off[m + 1];
     if (b1 < b0 || b0 < v.body_off[0] || b1 > v.body_off[v.n]) {       // not monotone: nothing is read through these offsets
         atomicOr(status, NUTSB_ST_BAD_OFFSETS);
-        slot_len[3 * m] = slot_len[3 * m + 1] = slot_len[3 * m + 2] = 0;
+        slot_len[3 * j] = slot_len[3 * j + 1] = slot_len[3 * j + 2] = 0;
         return;
     }
     const u32 blen = (u32)(b1 - b0);
     const u8 first = blen ? v.body[b0] : 0, last = blen ? v.body[b1 - 1] : 0;
-    const i32 room = v.user_room[spk] < v.n_rooms ? v.user_room[spk] : -1;
+    i32 who = spk, room;
+    bool home = true;
+    if (SHARD) home = nutsb_speech_home(v, sh, spk, &who, &room);
+    else room = v.user_room[spk] < v.n_rooms ? v.user_room[spk] : -1;
     for (u32 s = 0; s < 3; ++s) {
-        const SpeechSlot sl = nutsb_speech_slot(verb, s, spk, room, v.sflags[spk], v.ban_swearing != 0, first, last);
+        SpeechSlot sl = nutsb_speech_slot(verb, s, who, room, v.sflags[spk], v.ban_swearing != 0, first, last);
+        if (SHARD && !home) nutsb_speech_away(sl);
         u32 len = nutsb_speech_len(v, sl, spk, blen);
         if (len > NUTSB_MAX_TEXT) { atomicOr(status, NUTSB_ST_TEXT_TOO_LONG); len = 0; }
-        slot_len[3 * m + s] = len;
+        slot_len[3 * j + s] = len;
     }
 }
 
@@ -184,30 +253,37 @@ k_speech_measure(SpeechView v, u32 *slot_len, u32 *status)
 // piece write the op itself (kind, target, except, flags, gate).  Then the group copies the pieces one after
 // the other, all lanes on one piece.  (One warp per message with the rules evaluated op after op was 809
 // instructions per message, issue-bound at 0.92 ms for 1M lines.)
+// SHARD: one group per selected line j (line sel[j], ops 3j..3j+2; the gate stays the line's index in the batch).
 #define NUTSB_SPEECH_GROUP 16
+template <bool SHARD>
 __global__ void __launch_bounds__(256)
-k_speech_compose(SpeechView v, const u64 *text_off, u8 *text, u8 *kind, i32 *target, i32 *except_user, u8 *flags, i32 *gate)
+k_speech_compose(SpeechView v, SpeechShard sh, const u64 *text_off, u8 *text, u8 *kind, i32 *target, i32 *except_user, u8 *flags, i32 *gate)
 {
     constexpr int G = NUTSB_SPEECH_GROUP;
     const int lane = threadIdx.x & 31, gl = lane % G, g0 = lane - gl;
-    const i64 m = ((i64)blockIdx.x * blockDim.x + threadIdx.x) / G;
-    const bool have = m < v.n;
+    const i64 j = ((i64)blockIdx.x * blockDim.x + threadIdx.x) / G;
+    const bool have = j < (SHARD ? sh.k : v.n);
     // -- piece gl of message m (lane 15 has none)
     const u32 s = (u32)gl / 5u, part = (u32)gl % 5u;
     const u8 *src = nullptr; u32 len = 0; u8 *dst = nullptr;
     if (have && gl < 15) {
+        const i64 m = SHARD ? (i64)sh.sel[j] : j;
         const i32 spk = v.speaker[m];
         const u32 verb = v.verb[m];
         const bool ok = spk >= 0 && spk < v.n_users && verb < NUTSB_SPEECH_VERBS;
         const u64 b0 = v.body_off[m], b1 = v.body_off[m + 1];
         const u32 blen = (u32)(b1 - b0);
         const u8 first = blen ? v.body[b0] : 0, last = blen ? v.body[b1 - 1] : 0;
-        const i32 room = ok ? (v.user_room[spk] < v.n_rooms ? v.user_room[spk] : -1) : -1;
+        i32 who = spk, room = -1;
+        bool home = true;
+        if (SHARD) { if (ok) home = nutsb_speech_home(v, sh, spk, &who, &room); }   // (selected lines are valid)
+        else room = ok ? (v.user_room[spk] < v.n_rooms ? v.user_room[spk] : -1) : -1;
         const u32 sf = ok ? v.sflags[spk] : 0u;
-        const i64 q = 3 * m + s;
+        const i64 q = 3 * j + s;
         SpeechSlot sl{};
         sl.kind = NUTSB_OP_NONE; sl.target = -1; sl.except_user = -1;
-        if (ok) sl = nutsb_speech_slot(verb, s, spk, room, sf, v.ban_swearing != 0, first, last);
+        if (ok) sl = nutsb_speech_slot(verb, s, who, room, sf, v.ban_swearing != 0, first, last);
+        if (SHARD && !home) nutsb_speech_away(sl);
         const u64 o0 = text_off[q];
         const u32 slen = (u32)(text_off[q + 1] - o0);
         // (a composed line over NUTSB_MAX_TEXT was measured as 0 and flagged: dropped here)
