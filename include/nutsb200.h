@@ -294,7 +294,11 @@ int nutsb_set_user_names(nutsb_ctx *ctx, int32_t n_users, const uint8_t *names, 
 int nutsb_set_ban_swearing(nutsb_ctx *ctx, int on);
 /* n input lines: verb[n], speaker[n] (user index), bodies packed + off[n+1].  The device
  * runs contains_swearing on the bodies, composes the calls and renders them; streams as
- * for nutsb_write_batch.  *_dev: every pointer is a device pointer, streams stay in HBM. */
+ * for nutsb_write_batch.  *_dev: every pointer is a device pointer, streams stay in HBM.
+ * With nutsb_set_speech_record(ctx, 1) the three calls also record what say / emote / echo send to the
+ * room in its review buffer, as nutsb_q_speech does (see nutsb_set_speech_record); nutsb_speech_batch_dev
+ * then synchronises once more and returns with the records applied.  nutsb_timing of a speech batch describes its
+ * write pipeline: the composition and the recording step before it are in neither launches nor total_ms. */
 int nutsb_speech_batch(nutsb_ctx *ctx, int64_t n, const uint8_t *verb, const int32_t *speaker,
                        const uint8_t *bodies, const uint64_t *body_off, nutsb_streams *out);
 int nutsb_speech_batch_dev(nutsb_ctx *ctx, int64_t n, const uint8_t *verb, const int32_t *speaker,
@@ -305,6 +309,18 @@ int nutsb_speech_batch_iov(nutsb_ctx *ctx, int64_t n, const uint8_t *verb, const
 /* queue tier: one call of the reference's say()/shout()/... ; composed on the host, the swear
  * verdicts of the queued lines are taken in one device batch at nutsb_flush */
 int nutsb_q_speech(nutsb_ctx *ctx, int verb, int32_t user, const char *inpstr);
+/* 1: nutsb_speech_batch / _iov / _dev record what say / emote / echo send to the room, as nutsb_q_speech does.
+ * 0 (default): they leave the review buffers alone, as before.
+ * A line is recorded when its room line is sent: the speaker is in a room and not muzzled, and the line is not
+ * refused for swearing.  The record is the composed line as record() (c:2062) keeps it.  The records go in batch
+ * order after what the buffers held; the buffers change only when the whole call succeeds.  With record() calls
+ * still pending in the queue (nutsb_q_speech / nutsb_q_record since the last flush or review) the calls return
+ * NUTSB_E_STATE: flush first. */
+int nutsb_set_speech_record(nutsb_ctx *ctx, int on);
+/* Room `room`'s buffer as the reference holds it: REVIEW_LINES rows of REVIEW_LEN+2 bytes (rm->revbuff, strncpy's
+ * NUL padding included) and the ring position (rm->revline).  Records still pending in the queue are not in it
+ * until the next flush or review.  Either pointer may be NULL. */
+int nutsb_get_review_buffer(nutsb_ctx *ctx, int32_t room, uint8_t *rows, int32_t *line);
 
 /* ---- review buffers (queue tier; record c:2062, review c:5192, clear_revbuff c:2626) ------
  * nutsb_q_speech records what say / emote / echo send to the room (c:4099, c:4209, c:4304), as
@@ -427,6 +443,12 @@ int  nutsb_multi_speech_batch(nutsb_multi *m, int64_t n, const uint8_t *verb, co
                               const uint8_t *bodies, const uint64_t *body_off, nutsb_mstreams *out, int keep);
 int  nutsb_multi_speech_batch_iov(nutsb_multi *m, int64_t n, const uint8_t *verb, const int32_t *speaker,
                                   const uint8_t *bodies, const uint64_t *body_off, nutsb_miov_streams *out);
+/* Recording (nutsb_set_speech_record) on every shard: each records the lines of its own rooms, and the buffers change
+ * only when every shard has succeeded.  nutsb_multi_set_users carries each room's buffer to its new shard and local
+ * index.  Rank mode refuses it (NUTSB_E_UNSUPPORTED): a buffer cannot follow a room into another process.
+ * nutsb_multi_get_review_buffer: global room `room`'s buffer (nutsb_get_review_buffer). */
+int  nutsb_multi_set_speech_record(nutsb_multi *m, int on);
+int  nutsb_multi_get_review_buffer(nutsb_multi *m, int32_t room, uint8_t *rows, int32_t *line);
 
 /* ---- calls in flight on one device -----------------------------------------------------------------
  * A host-buffer call is H2D copy -> kernels -> D2H copy; PCIe is full duplex, so with two calls in flight one call's

@@ -33,6 +33,7 @@ SF_INVIS, SF_MUZZLED = 1, 2
 NEW, USER, WIZ, ARCH, GOD = 0, 1, 2, 3, 4
 
 E_INVAL, E_NOMEM, E_CUDA, E_UNSUPPORTED, E_RANGE, E_STATE = -1, -2, -3, -4, -5, -6
+REVIEW_LINES, REVIEW_LEN = 15, 200            # nuts333.h:37, :39 (NUTSB_REVIEW_LINES / NUTSB_REVIEW_LEN)
 
 u8p = C.POINTER(C.c_uint8)
 u64p = C.POINTER(C.c_uint64)
@@ -88,7 +89,7 @@ EXPORTS = [
     "nutsb_contains_swearing_batch", "nutsb_contains_swearing_batch_dev", "nutsb_site_banned_batch",
     "nutsb_site_banned_batch_dev", "nutsb_user_banned_batch", "nutsb_user_banned_batch_dev",
     "nutsb_set_user_names", "nutsb_set_ban_swearing", "nutsb_speech_batch", "nutsb_speech_batch_dev", "nutsb_speech_batch_iov", "nutsb_q_speech",
-    "nutsb_q_record", "nutsb_q_review", "nutsb_q_review_clear",
+    "nutsb_q_record", "nutsb_q_review", "nutsb_q_review_clear", "nutsb_set_speech_record", "nutsb_get_review_buffer",
     "nutsb_q_tell", "nutsb_q_pemote", "nutsb_q_wizshout", "nutsb_q_revtell",
     "nutsb_colour_com_count_batch", "nutsb_colour_com_strip_batch", "nutsb_stream_digests", "nutsb_q_write_user", "nutsb_q_write_room", "nutsb_q_write_room_except",
     "nutsb_q_write_level", "nutsb_q_write_sock", "nutsb_q_page_line", "nutsb_q_more", "nutsb_q_pending", "nutsb_flush", "nutsb_flush_iov", "nutsb_contains_swearing",
@@ -99,7 +100,7 @@ EXPORTS = [
     "nutsb_multi_route", "nutsb_multi_write_batch", "nutsb_multi_stream_digests", "nutsb_multi_contains_swearing_batch",
     "nutsb_multi_site_banned_batch", "nutsb_multi_user_banned_batch", "nutsb_multi_get_timing",
     "nutsb_multi_write_batch_iov", "nutsb_multi_shard_iov", "nutsb_multi_set_user_names", "nutsb_multi_set_ban_swearing",
-    "nutsb_multi_speech_batch", "nutsb_multi_speech_batch_iov",
+    "nutsb_multi_speech_batch", "nutsb_multi_speech_batch_iov", "nutsb_multi_set_speech_record", "nutsb_multi_get_review_buffer",
     "nutsb_pipe_create", "nutsb_pipe_destroy", "nutsb_pipe_depth", "nutsb_pipe_ctx", "nutsb_pipe_set_swear_words", "nutsb_pipe_set_users",
     "nutsb_pipe_set_user_names", "nutsb_pipe_set_ban_swearing", "nutsb_pipe_submit_speech_iov", "nutsb_pipe_submit_write_iov", "nutsb_pipe_wait",
 ]
@@ -142,6 +143,8 @@ def bind(lib: C.CDLL) -> C.CDLL:
     lib.nutsb_speech_batch_dev.argtypes = [vp, C.c_int64, vp, vp, vp, vp, C.POINTER(_Streams)]
     lib.nutsb_speech_batch_iov.argtypes = [vp, C.c_int64, vp, vp, vp, vp, C.POINTER(_IovStreams)]
     lib.nutsb_q_speech.argtypes = [vp, C.c_int, C.c_int32, C.c_char_p]
+    lib.nutsb_set_speech_record.argtypes = [vp, C.c_int]
+    lib.nutsb_get_review_buffer.argtypes = [vp, C.c_int32, vp, C.POINTER(C.c_int32)]
     lib.nutsb_set_clones.argtypes = [vp, C.c_int32, vp, vp]
     lib.nutsb_set_room_names.argtypes = [vp, C.c_int32, vp, vp]
     lib.nutsb_set_remotes.argtypes = [vp, C.c_int32, vp, vp]
@@ -196,6 +199,8 @@ def bind(lib: C.CDLL) -> C.CDLL:
     lib.nutsb_multi_set_ban_swearing.argtypes = [vp, C.c_int]
     lib.nutsb_multi_speech_batch.argtypes = [vp, C.c_int64, vp, vp, vp, vp, C.POINTER(_MStreams), C.c_int]
     lib.nutsb_multi_speech_batch_iov.argtypes = [vp, C.c_int64, vp, vp, vp, vp, C.POINTER(_MIovStreams)]
+    lib.nutsb_multi_set_speech_record.argtypes = [vp, C.c_int]
+    lib.nutsb_multi_get_review_buffer.argtypes = [vp, C.c_int32, vp, C.POINTER(C.c_int32)]
     lib.nutsb_pipe_create.argtypes = [C.POINTER(vp), C.c_int, C.c_int]
     lib.nutsb_pipe_destroy.argtypes = [vp]
     lib.nutsb_pipe_destroy.restype = None
@@ -303,6 +308,14 @@ class IovStreams:
         return Streams(self.off.copy(), data, self.n_deliveries)
 
 
+def _review_buffer(fn, h, room, ck):
+    buf = (C.c_uint8 * (REVIEW_LINES * (REVIEW_LEN + 2)))()
+    line = C.c_int32(0)
+    ck(fn(h, room, buf, C.byref(line)))
+    raw = bytes(buf)
+    return [raw[i * (REVIEW_LEN + 2):(i + 1) * (REVIEW_LEN + 2)] for i in range(REVIEW_LINES)], line.value
+
+
 class Context:
     """One context per GPU (nutsb_create / nutsb_destroy)."""
 
@@ -380,6 +393,15 @@ class Context:
         self._ck(self.lib.nutsb_speech_batch_iov(self._h, len(verb), _addr(verb), _addr(speaker),
                                                  _addr(bodies) if bodies.size else None, _addr(body_off), C.byref(st)))
         return self._host_iov(st)
+
+    def set_speech_record(self, on: bool):
+        """on: speech batches record what say / emote / echo send to the room in its review buffer, as the queue
+        tier does (nutsb_set_speech_record)"""
+        self._ck(self.lib.nutsb_set_speech_record(self._h, 1 if on else 0))
+
+    def review_buffer(self, room):
+        """-> (rows, line): the room's REVIEW_LINES rows of REVIEW_LEN + 2 bytes each and the ring position"""
+        return _review_buffer(self.lib.nutsb_get_review_buffer, self._h, room, self._ck)
 
     def set_clones(self, owner, hear):
         owner, hear = _np(owner, np.int32), _np(hear, np.uint8)
@@ -838,6 +860,14 @@ class MultiContext:
         st = _MIovStreams()
         self._ck(self.lib.nutsb_multi_speech_batch_iov(self._h, *args, C.byref(st)))
         return MIovStreams(st)
+
+    def set_speech_record(self, on: bool):
+        """Context.set_speech_record on every shard (refused in rank mode)"""
+        self._ck(self.lib.nutsb_multi_set_speech_record(self._h, 1 if on else 0))
+
+    def review_buffer(self, room):
+        """-> (rows, line) of global room `room` (Context.review_buffer)"""
+        return _review_buffer(self.lib.nutsb_multi_get_review_buffer, self._h, room, self._ck)
 
     def stream_digests(self, digest=None):
         """Per-user digests in global order; digest given: the fold continues from it (chunked jobs)."""

@@ -171,6 +171,10 @@ struct nutsb_ctx {
     std::vector<TellBuf> revtell;                                // per user (nuts333.h:73)
     std::vector<RevBuf> rev;
     std::vector<PendingRec> q_rec;                               // record() calls whose line may still be refused (swearing)
+    // the speech batch's records (nutsb_set_speech_record): k_speech_rec_* scratch, the packed records on the host
+    bool speech_record = false, rec_ready = false; u64 rec_total = 0;
+    DBuf d_rec_key, d_rec_line, d_rec_k[2], d_rec_v[2], d_rec_cnt, d_rec_seg, d_rec_lens, d_rec_bytes, d_rec_off, d_rec_out;
+    HBuf h_rec;
 };
 
 static int fail(nutsb_ctx *c, int code, const char *fmt, const char *a = "")
@@ -235,6 +239,12 @@ struct OutSel {
     __device__ void operator()(i64 i, u64 ex) const { if (i == n) sel[n] = (i32)ex; else if (keep[i]) sel[ex] = (i32)i; }
 };
 struct OutU64 { u64 *p; __device__ void operator()(i64 i, u64 ex) const { p[i] = ex; } };
+// the speech batch's records (k_speech_rec_mark's keys): the marked lines' rooms and indices in order, their number
+struct InRecKey { const u32 *key; __device__ u64 operator()(i64 i) const { return key[i] != NUTSB_REC_NONE; } };
+struct OutRec {
+    const u32 *key; u32 *room, *line, *count; i64 n;
+    __device__ void operator()(i64 i, u64 ex) const { if (i == n) *count = (u32)ex; else if (key[i] != NUTSB_REC_NONE) { room[ex] = key[i]; line[ex] = (u32)i; } }
+};
 struct InEntryPacked {
     const u8 *info;
     __device__ u64 operator()(i64 i) const { const u32 f = info[i]; return (u64)(f & 1u) | ((u64)((f >> 1) != 0) << 32); }
@@ -492,10 +502,12 @@ NUTSB_API void nutsb_destroy(nutsb_ctx *c)
         &c->d_names, &c->d_name_off, &c->d_sflags, &c->d_lit, &c->d_lit_off, &c->d_sp_len, &c->d_sp_off, &c->d_sp_text,
         &c->d_sp_kind, &c->d_sp_target, &c->d_sp_except, &c->d_sp_flags, &c->d_sp_gate, &c->d_sp_verdict,
         &c->s_verb, &c->s_speaker, &c->s_body, &c->s_boff,
-        &c->d_g_user_shard, &c->d_g_user_local, &c->d_g_has_room, &c->d_g_names, &c->d_g_name_off, &c->d_g_sflags, &c->d_sp_keep, &c->d_sp_sel };
+        &c->d_g_user_shard, &c->d_g_user_local, &c->d_g_has_room, &c->d_g_names, &c->d_g_name_off, &c->d_g_sflags, &c->d_sp_keep, &c->d_sp_sel,
+        &c->d_rec_key, &c->d_rec_line, &c->d_rec_k[0], &c->d_rec_k[1], &c->d_rec_v[0], &c->d_rec_v[1], &c->d_rec_cnt, &c->d_rec_seg,
+        &c->d_rec_lens, &c->d_rec_bytes, &c->d_rec_off, &c->d_rec_out };
     for (DBuf *b : all) release(*b);
     release(c->h_small); release(c->h_off); release(c->h_out);
-    release(c->h_dir); release(c->h_iov); release(c->h_iov_first); release(c->h_iov_cnt);
+    release(c->h_dir); release(c->h_iov); release(c->h_iov_first); release(c->h_iov_cnt); release(c->h_rec);
     for (auto &e : c->ev) if (e) cudaEventDestroy(e);
     for (auto &e : c->dep) if (e) cudaEventDestroy(e);
     if (c->side) { cudaStreamSynchronize(c->side); cudaStreamDestroy(c->side); }
@@ -2043,6 +2055,91 @@ NUTSB_API int nutsb_q_revtell(nutsb_ctx *c, int32_t user)
     return nutsb_q_write_user(c, user, "\n~BB~FG*** End ***\n\n");
 }
 
+// The records of a composed speech batch (k lines, ops 3j..3j+2 in d_sp_*, verdicts in d_sp_verdict), packed in
+// d_rec_out (nutsb_speech.cuh); their size goes to h_small at byte 2048, which run_write's synchronisations make
+// readable.  On the main stream: the scans and the sort share its scan state with run_write's planning.
+static int speech_records(nutsb_ctx *c, i64 k, const u8 *verb, const SpeechShard &sh, bool shard)
+{
+    cudaStream_t st = c->stream;
+    const u32 R = (u32)c->R;
+    u64 *h_total = c->h_small.as<u64>() + 256;
+    if (R == 0 || k == 0) { *h_total = 0; return NUTSB_OK; }
+    const size_t kk = (size_t)k;
+    TRY(ensure(c, c->d_rec_key, kk * 4)); TRY(ensure(c, c->d_rec_line, kk * 4)); TRY(ensure(c, c->d_rec_cnt, 16));
+    for (int q = 0; q < 2; ++q) { TRY(ensure(c, c->d_rec_k[q], kk * 4 + 16)); TRY(ensure(c, c->d_rec_v[q], kk * 4 + 16)); }   // radix_sort's sizes
+    TRY(ensure(c, c->d_rec_seg, ((size_t)R + 1) * 4)); TRY(ensure(c, c->d_rec_lens, (size_t)R * 16));
+    TRY(ensure(c, c->d_rec_bytes, (size_t)R * 4)); TRY(ensure(c, c->d_rec_off, ((size_t)R + 1) * 8));
+    const size_t rooms = std::min<size_t>(R, kk), lines = std::min<size_t>(kk, (size_t)R * NUTSB_REVIEW_LINES);
+    TRY(ensure(c, c->d_rec_out, rooms * NUTSB_REC_HEAD + lines * NUTSB_REVIEW_LEN + 16));
+    u32 *key = c->d_rec_key.as<u32>(), *line = c->d_rec_line.as<u32>(), *cnt = c->d_rec_cnt.as<u32>();
+    if (shard) { NUTSB_LAUNCH(cdiv(kk, 256), 256, st, k_speech_rec_mark<true>, verb, sh, k, c->d_sp_kind.as<u8>(), c->d_sp_target.as<i32>(), c->d_sp_gate.as<i32>(), c->d_sp_verdict.as<u8>(), key); }
+    else       { NUTSB_LAUNCH(cdiv(kk, 256), 256, st, k_speech_rec_mark<false>, verb, sh, k, c->d_sp_kind.as<u8>(), c->d_sp_target.as<i32>(), c->d_sp_gate.as<i32>(), c->d_sp_verdict.as<u8>(), key); }
+    CKL();
+    TRY(run_scan(c, InRecKey{key}, OutRec{key, c->d_rec_k[0].as<u32>(), line, cnt, k}, k, nullptr));
+    u32 *keys = nullptr, *vals = nullptr;
+    TRY(radix_sort(c, c->d_rec_k, c->d_rec_v, k, cnt, bits_for(R), &keys, &vals));
+    u32 *seg = c->d_rec_seg.as<u32>();
+    NUTSB_LAUNCH(cdiv(kk + 1, 256), 256, st, k_speech_rec_bounds, keys, cnt, k, R, seg); CKL();
+    NUTSB_LAUNCH(cdiv((u64)R * 32, 256), 256, st, k_speech_rec_tail, seg, vals, line, c->d_sp_off.as<u64>(), c->d_sp_text.as<u8>(), R,
+                 c->d_rec_lens.as<u8>(), c->d_rec_bytes.as<u32>()); CKL();
+    TRY(run_scan(c, InU32{c->d_rec_bytes.as<u32>()}, OutU64{c->d_rec_off.as<u64>()}, (i64)R, nullptr));
+    NUTSB_LAUNCH(cdiv((u64)R * 32, 256), 256, st, k_speech_rec_pack, seg, vals, line, c->d_sp_off.as<u64>(), c->d_sp_text.as<u8>(), R,
+                 c->d_rec_lens.as<u8>(), c->d_rec_off.as<u64>(), c->d_rec_out.as<u8>()); CKL();
+    CK(cudaMemcpyAsync(h_total, c->d_rec_off.as<u64>() + R, 8, cudaMemcpyDeviceToHost, st));
+    return NUTSB_OK;
+}
+
+// The packed records to the host (h_rec) once run_write has synchronised: one copy of the bytes they keep.
+static int fetch_records(nutsb_ctx *c)
+{
+    CK(cudaStreamSynchronize(c->stream));
+    const u64 total = c->h_small.as<u64>()[256];
+    TRY(ensure_host(c, c->h_rec, (size_t)total + 16));
+    if (total) {
+        CK(cudaMemcpyAsync(c->h_rec.p, c->d_rec_out.p, (size_t)total, cudaMemcpyDeviceToHost, c->stream));
+        CK(cudaStreamSynchronize(c->stream));
+    }
+    c->rec_total = total; c->rec_ready = true;
+    return NUTSB_OK;
+}
+
+// ... and into the rings: room r's c records end at (line + c) % REVIEW_LINES, the last min(c, REVIEW_LINES) of them
+// where record() would have put them (do_record: strncpy's NUL padding, '\n' at REVIEW_LEN).
+static void apply_records(nutsb_ctx *c)
+{
+    const u8 *p = c->h_rec.as<u8>(), *end = p + c->rec_total;
+    while (p < end) {
+        u32 room, cnt;
+        memcpy(&room, p, 4); memcpy(&cnt, p + 4, 4);
+        const u8 *lens = p + 8;
+        const u32 t = std::min<u32>(cnt, NUTSB_REVIEW_LINES);
+        const u8 *text = p + NUTSB_REC_HEAD;
+        nutsb_ctx::RevBuf &rb = c->rev[room];
+        for (u32 i = 0; i < t; ++i) {
+            char *row = rb.buf[(rb.line + (cnt - t) + i) % NUTSB_REVIEW_LINES];
+            memset(row, 0, NUTSB_REVIEW_LEN);
+            memcpy(row, text, lens[i]);
+            row[NUTSB_REVIEW_LEN] = '\n'; row[NUTSB_REVIEW_LEN + 1] = '\0';
+            text += lens[i];
+        }
+        rb.line = (int)((rb.line + cnt) % NUTSB_REVIEW_LINES);
+        p = text;
+    }
+    c->rec_ready = false;
+}
+
+NUTSB_API int nutsb_set_speech_record(nutsb_ctx *c, int on) { if (!c) return NUTSB_E_INVAL; c->speech_record = on != 0; return NUTSB_OK; }
+
+NUTSB_API int nutsb_get_review_buffer(nutsb_ctx *c, int32_t room, uint8_t *rows, int32_t *line)
+{
+    if (!c) return NUTSB_E_INVAL;
+    if (room < 0 || room >= (i32)c->rev.size()) return fail(c, NUTSB_E_RANGE, "room index out of range%s");
+    const nutsb_ctx::RevBuf &rb = c->rev[(size_t)room];
+    if (rows) memcpy(rows, rb.buf, sizeof rb.buf);
+    if (line) *line = rb.line;
+    return NUTSB_OK;
+}
+
 // shard: the context is one shard of a nutsb_multi, the speakers are global user indices, and only the lines
 // that produce an op on this shard are composed (k_speech_route, then a scan compacts their indices)
 static int run_speech(nutsb_ctx *c, i64 n, const u8 *verb, const i32 *speaker, const u8 *bodies, const u64 *body_off, nutsb_streams *out,
@@ -2051,6 +2148,7 @@ static int run_speech(nutsb_ctx *c, i64 n, const u8 *verb, const i32 *speaker, c
     TRY(speech_ready(c));
     if (shard && (!c->have_g_names || c->shard < 0)) return fail(c, NUTSB_E_STATE, "nutsb_multi_set_user_names does not match the population%s");
     cudaStream_t st = c->stream;
+    c->h_small.as<u64>()[256] = 0;                             // no records until speech_records says otherwise
     if (n == 0) { nutsb_ops o{}; return run_write(c, &o, out, iv); }
     SpeechView v{ n, verb, speaker, bodies, body_off, c->d_names.as<u8>(), c->d_name_off.as<u64>(), c->d_sflags.as<u8>(),
                   c->d_user_room.as<i32>(), c->d_lit.as<u8>(), c->d_lit_off.as<u32>(), c->U, c->R, c->ban_swearing ? 1u : 0u };
@@ -2103,6 +2201,7 @@ static int run_speech(nutsb_ctx *c, i64 n, const u8 *verb, const i32 *speaker, c
     CKL();
     // the verdicts of every line: a shard delivers gated shouts of speakers who live elsewhere (the gates are line indices)
     TRY(verdict_dev(c, V_SWEAR, n, bodies, body_off, c->d_sp_verdict.as<u8>()));
+    if (c->speech_record) TRY(speech_records(c, k, verb, sh, shard));
     nutsb_ops o{ (i64)k3, c->d_sp_text.as<u8>(), c->d_sp_off.as<u64>(), c->d_sp_kind.as<u8>(), c->d_sp_target.as<i32>(),
                  c->d_sp_except.as<i32>(), c->d_sp_flags.as<u8>(), c->d_sp_gate.as<i32>(), c->d_sp_verdict.as<u8>() };
     return run_write(c, &o, out, iv);
@@ -2131,11 +2230,17 @@ static int speech_batch(nutsb_ctx *c, i64 n, const u8 *verb, const i32 *speaker,
                         bool upload, const Result &r, bool shard = false)
 {
     if (!c || (!r.st && !r.iov) || n < 0 || (n && (!verb || !speaker || !body_off))) return fail(c, NUTSB_E_INVAL, "bad argument%s");
+    c->rec_ready = false;
+    if (c->speech_record && !c->q_rec.empty())
+        return fail(c, NUTSB_E_STATE, "record() calls are pending in the queue: flush first%s");
     TRY(begin_write(c, false));
     if (upload) TRY(upload_speech(c, n, verb, speaker, bodies, body_off));
     nutsb_streams ds{}; IovReq iv;
     TRY(run_speech(c, n, verb, speaker, bodies, body_off, &ds, r.form == Result::IOV ? &iv : nullptr, shard));
-    return deliver(c, upload, ds, iv, r);
+    if (c->speech_record) TRY(fetch_records(c));             // before the result is handed over: an error leaves it untouched
+    TRY(deliver(c, upload, ds, iv, r));
+    if (c->speech_record && !shard) apply_records(c);          // (nutsb_multi applies every shard's once all have succeeded)
+    return NUTSB_OK;
 }
 
 NUTSB_API int nutsb_speech_batch_dev(nutsb_ctx *c, int64_t n, const uint8_t *verb, const int32_t *speaker,

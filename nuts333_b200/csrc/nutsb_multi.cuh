@@ -28,6 +28,7 @@
 
 struct nutsb_multi {
     int n_shards = 0;
+    bool rank = false;                            // nutsb_multi_create_rank: this process runs one shard
     std::vector<nutsb_ctx *> ctx;                 // [n_shards], null = not run by this process
     std::string err;
     // plan
@@ -46,6 +47,9 @@ struct nutsb_multi {
     std::vector<u64> len; std::vector<const u8 *> ptr;
     std::vector<const nutsb_iovec *> iov; std::vector<u32> count;
     std::vector<u64> dg_local;
+    // every room's review buffer in global order, taken from the last plan that was set up whole, until a re-plan
+    // succeeds (one that fails half way has already reshaped some shards' buffers: its retry starts from these)
+    std::vector<nutsb_ctx::RevBuf> rev_carry; bool carry = false;
 };
 
 static int mfail(nutsb_multi *m, int code, const char *msg) { if (m) m->err = msg; return code; }
@@ -68,6 +72,7 @@ static int multi_create(nutsb_multi **out, int n_shards, const int *device_ids, 
     nutsb_multi *m = new (std::nothrow) nutsb_multi;
     if (!m) return NUTSB_E_NOMEM;
     m->n_shards = n_shards;
+    m->rank = only_shard >= 0;
     m->ctx.assign((size_t)n_shards, nullptr);
     m->routed.resize((size_t)n_shards);
     for (int s = 0; s < n_shards; ++s) {
@@ -177,6 +182,21 @@ NUTSB_API int nutsb_multi_set_users(nutsb_multi *m, int32_t n_users, int32_t n_r
             return mfail(m, NUTSB_E_UNSUPPORTED, "clones / remote users: their relays cross rooms (and shards); use one context");
     }
     const int S = m->n_shards;
+    // queued ops name users by index (nutsb_set_users refuses them): checked on every shard before anything changes
+    for (nutsb_ctx *c : m->ctx)
+        if (c && (c->q.n() || !c->q_rec.empty()))
+            return mfail(m, NUTSB_E_STATE, "nutsb_multi_set_users with ops still queued on a shard: flush first");
+    // every room's review buffer as the old plan holds it (on a shard this process runs), to follow the room to its
+    // new shard and local index; a room new to the population starts empty, as on one context
+    if (m->have_users) {
+        m->rev_carry.assign((size_t)m->R, nutsb_ctx::RevBuf{});
+        for (i32 r = 0; r < m->R; ++r) {
+            const nutsb_ctx *c = m->ctx[(size_t)m->room_shard[(size_t)r]];
+            const size_t l = (size_t)m->room_local[(size_t)r];
+            if (c && l < c->rev.size()) m->rev_carry[(size_t)r] = c->rev[l];
+        }
+        m->carry = true;
+    }
     m->have_users = false; m->U = n_users; m->R = n_rooms;
     std::vector<u64> pop((size_t)n_rooms, 0);
     for (i32 u = 0; u < n_users; ++u) if (room[u] >= 0) pop[(size_t)room[u]]++;
@@ -217,6 +237,10 @@ NUTSB_API int nutsb_multi_set_users(nutsb_multi *m, int32_t n_users, int32_t n_r
         if (rc == NUTSB_OK) rc = shard_tables(c, s, m, room);
         if (rc != NUTSB_OK) { m->err = nutsb_last_error(c); return rc; }
     }
+    for (i32 r = 0; r < n_rooms; ++r)
+        if (nutsb_ctx *c = m->ctx[(size_t)m->room_shard[(size_t)r]])
+            c->rev[(size_t)m->room_local[(size_t)r]] = m->carry && (size_t)r < m->rev_carry.size() ? m->rev_carry[(size_t)r] : nutsb_ctx::RevBuf{};
+    m->rev_carry.clear(); m->carry = false;
     m->len.assign((size_t)n_users, 0); m->ptr.assign((size_t)n_users, nullptr);
     m->iov.assign((size_t)n_users, nullptr); m->count.assign((size_t)n_users, 0);
     m->have_users = true;
@@ -360,10 +384,35 @@ static int multi_speech(nutsb_multi *m, i64 n, const u8 *verb, const i32 *speake
 {
     if (!m->have_users) return mfail(m, NUTSB_E_STATE, "nutsb_multi_set_users has not been called");
     if (!m->have_names || (i32)m->sflags.size() != m->U) return mfail(m, NUTSB_E_STATE, "nutsb_multi_set_user_names does not match the population");
-    return multi_batch(m, form, [=](nutsb_ctx *c, nutsb_multi::Routed &r) {
+    TRY(multi_batch(m, form, [=](nutsb_ctx *c, nutsb_multi::Routed &r) {
         const Result res = form == M_IOV ? Result{ Result::IOV, nullptr, &r.iov } : Result{ form == M_KEEP ? Result::HBM : Result::HOST, &r.out, nullptr };
         return speech_batch(c, n, verb, speaker, bodies, body_off, true, res, true);
-    }, ms, mi);
+    }, ms, mi));
+    for (nutsb_ctx *c : m->ctx) if (c && c->rec_ready) apply_records(c);      // every shard has succeeded: all or nothing
+    return NUTSB_OK;
+}
+
+// Recording (nutsb_set_speech_record) on every shard: each records its own rooms.  Not in rank mode: a room's buffer
+// could not follow it to a shard another process runs.
+NUTSB_API int nutsb_multi_set_speech_record(nutsb_multi *m, int on)
+{
+    if (!m) return NUTSB_E_INVAL;
+    if (on && m->rank) return mfail(m, NUTSB_E_UNSUPPORTED, "speech records in rank mode: a room's review buffer cannot follow it to another process");
+    MEACH(nutsb_set_speech_record(c_, on));
+    return NUTSB_OK;
+}
+
+// Global room `room`'s buffer (nutsb_get_review_buffer), from the shard that holds the room.
+NUTSB_API int nutsb_multi_get_review_buffer(nutsb_multi *m, int32_t room, uint8_t *rows, int32_t *line)
+{
+    if (!m) return NUTSB_E_INVAL;
+    if (!m->have_users) return mfail(m, NUTSB_E_STATE, "nutsb_multi_set_users has not been called");
+    if (room < 0 || room >= m->R) return mfail(m, NUTSB_E_RANGE, "room index out of range");
+    nutsb_ctx *c = m->ctx[(size_t)m->room_shard[(size_t)room]];
+    if (!c) return mfail(m, NUTSB_E_UNSUPPORTED, "the room lives on a shard another process runs");
+    const int rc = nutsb_get_review_buffer(c, m->room_local[(size_t)room], rows, line);
+    if (rc != NUTSB_OK) m->err = nutsb_last_error(c);
+    return rc;
 }
 
 NUTSB_API int nutsb_multi_speech_batch(nutsb_multi *m, int64_t n, const uint8_t *verb, const int32_t *speaker,

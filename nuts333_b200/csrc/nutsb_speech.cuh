@@ -14,6 +14,7 @@
 // nutsb_q_speech) and the batch tier (device composer, k_speech_*) cannot drift apart.
 #pragma once
 #include "nutsb_common.cuh"
+#include "nutsb_kernels.cuh"          // nutsb_seg_bounds
 
 #define NUTSB_SPEECH_SAY    0
 #define NUTSB_SPEECH_SHOUT  1
@@ -325,5 +326,95 @@ k_speech_compose(SpeechView v, SpeechShard sh, const u64 *text_off, u8 *text, u8
         const u8 *ps = (const u8 *)(size_t)__shfl_sync(NUTSB_FULL, (u64)(size_t)src, g0 + i);
         u8 *pd = (u8 *)(size_t)__shfl_sync(NUTSB_FULL, (u64)(size_t)dst, g0 + i);
         for (u32 k = (u32)gl; k < n; k += G) pd[k] = ps[k];
+    }
+}
+
+// ---- recording (nutsb_set_speech_record): record(user->room, text) of say / emote / echo ----------------------
+// c:4099, c:4209, c:4304.  The lines a batch records in a room go into its ring in batch order, so only the last
+// REVIEW_LINES of each room can survive the batch, and of each only what strncpy keeps: its first REVIEW_LEN bytes,
+// up to an embedded NUL.  The steps, all on the context's main stream (the scans and the sort share its scan state):
+//   k_speech_rec_mark    key[j] = the room composed line j records in, or NUTSB_REC_NONE
+//   scan (compaction)    the marked lines' rooms and line indices, in batch order, and their number
+//   radix sort by room   stable: batch order within a room
+//   k_speech_rec_bounds  seg[r] .. seg[r+1]: room r's records in the sorted order
+//   k_speech_rec_tail    per room: the bytes strncpy keeps of its last min(c, REVIEW_LINES) records
+//   scan over the rooms  where each room's record lands in the packed buffer
+//   k_speech_rec_pack    per room that recorded anything:  u32 room | u32 c | u8 len[16] | the kept bytes, line after line
+// The host copies the packed buffer once and applies it to the rings after the batch has been delivered.
+#define NUTSB_REC_NONE 0xffffffffu
+#define NUTSB_REC_HEAD 24u
+
+// One thread per composed line j (line sel[j] of the batch in shard mode; its ops are 3j..3j+2).  Recorded: say,
+// emote and echo whose room op (slot 2) is live with a room -- not muzzled, in a room, on the speaker's own shard --
+// and not refused for swearing.
+template <bool SHARD>
+__global__ void __launch_bounds__(256)
+k_speech_rec_mark(const u8 *verb, SpeechShard sh, i64 k, const u8 *kind, const i32 *target, const i32 *gate, const u8 *verdict, u32 *key)
+{
+    const i64 j = (i64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= k) return;
+    const i64 m = SHARD ? (i64)sh.sel[j] : j;
+    const u32 v = verb[m];
+    const i64 q = 3 * j + 2;
+    const i32 g = gate[q];
+    const bool rec = (v == NUTSB_SPEECH_SAY || v == NUTSB_SPEECH_EMOTE || v == NUTSB_SPEECH_ECHO)
+                     && kind[q] == NUTSB_OP_ROOM && target[q] >= 0 && (g < 0 || !verdict[g]);
+    key[j] = rec ? (u32)target[q] : NUTSB_REC_NONE;
+}
+
+// Thread i in [0, k]: the room bounds of the *n_rec sorted keys (seg[0..n_rooms]).
+__global__ void __launch_bounds__(256)
+k_speech_rec_bounds(const u32 *keys, const u32 *n_rec, i64 k, u32 n_rooms, u32 *seg)
+{
+    const i64 i = (i64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i > k) return;
+    nutsb_seg_bounds(keys, (i64)*n_rec, i, n_rooms, seg);
+}
+
+// One warp per room, lane i on the room's i-th kept record: how many bytes strncpy takes of it.  vals[] = the sorted
+// records' positions in line[] (the composed line indices in batch order).  bytes[r] = room r's size in the packed
+// buffer (0: nothing recorded there).
+__global__ void __launch_bounds__(256)
+k_speech_rec_tail(const u32 *seg, const u32 *vals, const u32 *line, const u64 *text_off, const u8 *text, u32 n_rooms,
+                  u8 *lens, u32 *bytes)
+{
+    const i64 r = ((i64)blockIdx.x * blockDim.x + threadIdx.x) / 32;
+    const u32 lane = threadIdx.x & 31;
+    if (r >= n_rooms) return;                                   // (the whole warp)
+    const u32 b = seg[r + 1], c = b - seg[r], t = c < NUTSB_REVIEW_LINES ? c : NUTSB_REVIEW_LINES;
+    u32 len = 0;
+    if (lane < t) {
+        const u64 q = 3ull * line[vals[b - t + lane]] + 2;
+        const u64 o0 = text_off[q], o1 = text_off[q + 1];
+        const u32 lim = o1 - o0 < NUTSB_REVIEW_LEN ? (u32)(o1 - o0) : NUTSB_REVIEW_LEN;
+        const u8 *p = text + o0;
+        while (len < lim && p[len]) ++len;
+        lens[16 * r + lane] = (u8)len;
+    }
+    for (int d = 16; d; d >>= 1) len += __shfl_xor_sync(NUTSB_FULL, len, d);
+    if (lane == 0) bytes[r] = c ? NUTSB_REC_HEAD + len : 0;
+}
+
+// One warp per room that recorded anything: its header and kept bytes at out + off[r].
+__global__ void __launch_bounds__(256)
+k_speech_rec_pack(const u32 *seg, const u32 *vals, const u32 *line, const u64 *text_off, const u8 *text, u32 n_rooms,
+                  const u8 *lens, const u64 *off, u8 *out)
+{
+    const i64 r = ((i64)blockIdx.x * blockDim.x + threadIdx.x) / 32;
+    const u32 lane = threadIdx.x & 31;
+    if (r >= n_rooms) return;
+    const u32 b = seg[r + 1], c = b - seg[r], t = c < NUTSB_REVIEW_LINES ? c : NUTSB_REVIEW_LINES;
+    if (c == 0) return;
+    u8 *dst = out + off[r];
+    if (lane < NUTSB_REC_HEAD) {
+        const u32 w = lane < 4 ? (u32)r : c;
+        dst[lane] = lane < 8 ? (u8)(w >> (8 * (lane & 3))) : (lane - 8 < t ? lens[16 * r + lane - 8] : (u8)0);
+    }
+    dst += NUTSB_REC_HEAD;
+    for (u32 i = 0; i < t; ++i) {
+        const u32 n = lens[16 * r + i];
+        const u8 *src = text + text_off[3ull * line[vals[b - t + i]] + 2];
+        for (u32 x = lane; x < n; x += 32) dst[x] = src[x];
+        dst += n;
     }
 }
