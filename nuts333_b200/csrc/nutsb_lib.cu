@@ -23,12 +23,19 @@
 // ---------------------------------------------------------------------------------------
 // buffers
 // ---------------------------------------------------------------------------------------
+// Each owns its memory and frees it when destroyed: nutsb_destroy makes the context's device current first.
 struct DBuf {                        // growable device buffer
     void *p = nullptr; size_t cap = 0;
+    DBuf() = default;
+    DBuf(const DBuf &) = delete; DBuf &operator=(const DBuf &) = delete;
+    ~DBuf() { if (p) cudaFree(p); }
     template <class T> T *as() const { return (T *)p; }
 };
 struct HBuf {                        // growable pinned host buffer
     void *p = nullptr; size_t cap = 0;
+    HBuf() = default;
+    HBuf(const HBuf &) = delete; HBuf &operator=(const HBuf &) = delete;
+    ~HBuf() { if (p) cudaFreeHost(p); }
     template <class T> T *as() const { return (T *)p; }
 };
 
@@ -78,6 +85,22 @@ struct HostOps {
         o.target = target.empty() ? &z32 : target.data(); o.except_user = except.empty() ? &z32 : except.data();
         if (verdict) { o.gate = gate.empty() ? &z32 : gate.data(); o.verdict = verdict; }
         return o;
+    }
+};
+
+// A review buffer as the reference keeps it (a room's, nuts333.h:95; a user's revtell, nuts333.h:73): N rows of
+// REVIEW_LEN+2 bytes, `line` the next row to write.  nutsb_get_review_buffer hands `buf` out as it stands.
+template <int N> struct ReviewRing {
+    char buf[N][NUTSB_REVIEW_LEN + 2]; int line;
+    // one row as record() (c:2062) / record_tell() (c:2074) write it, given the len <= REVIEW_LEN bytes their
+    // strncpy keeps: those bytes, NUL padding up to REVIEW_LEN, '\n', NUL
+    void put(const void *bytes, size_t len)
+    {
+        char *row = buf[line];
+        memcpy(row, bytes, len);
+        memset(row + len, 0, NUTSB_REVIEW_LEN - len);
+        row[NUTSB_REVIEW_LEN] = '\n'; row[NUTSB_REVIEW_LEN + 1] = '\0';
+        line = (line + 1) % N;
     }
 };
 
@@ -134,9 +157,9 @@ struct nutsb_ctx {
     DBuf d_bl_op, d_bl_room, d_evk[2], d_evv[2], d_ev_ukey, d_ev_delta, d_ev_op;
     DBuf d_sv_ukey, d_sv_delta, d_sv_op, d_sv_pre, d_ev_off;
     DBuf d_vp_on, d_vp_off, d_cp;
-    DBuf d_room_tile_off, d_room_cell_off, d_room_item_off, d_sizes, d_counters;
+    DBuf d_room_tile_off, d_room_cell_off, d_room_item_off, d_counters;
     DBuf d_runs, d_items, d_slab, d_bl_meta, d_slots;
-    DBuf d_off, d_out, d_digest, d_ulen;
+    DBuf d_off, d_out, d_digest;
     DBuf d_dpre, d_dir, d_iov, d_iov_first, d_iov_cnt;           // gather-list mode (nutsb_write_batch_iov)
     HBuf h_small, h_off, h_out, h_dir, h_iov, h_iov_first, h_iov_cnt;
     u64 last_total = 0; bool have_streams = false;
@@ -164,12 +187,10 @@ struct nutsb_ctx {
     std::vector<u8> q_sw_text; std::vector<u64> q_sw_off{0};     // bodies whose swear verdict gates queued ops
     std::vector<u8> q_sw_verdict;                                // ... their verdicts, once taken (flush / review)
 
-    // review buffers (nuts333.h:95, REVIEW_LINES x REVIEW_LEN+2 per room), host state of the queue tier
-    struct RevBuf { char buf[NUTSB_REVIEW_LINES][NUTSB_REVIEW_LEN + 2]; int line; };
+    // review buffers, host state of the queue tier
     struct PendingRec { i32 room, gate; std::string text; };
-    struct TellBuf { char buf[NUTSB_REVTELL_LINES][NUTSB_REVIEW_LEN + 2]; int line; };
-    std::vector<TellBuf> revtell;                                // per user (nuts333.h:73)
-    std::vector<RevBuf> rev;
+    std::vector<ReviewRing<NUTSB_REVTELL_LINES>> revtell;        // per user
+    std::vector<ReviewRing<NUTSB_REVIEW_LINES>> rev;             // per room
     std::vector<PendingRec> q_rec;                               // record() calls whose line may still be refused (swearing)
     // the speech batch's records (nutsb_set_speech_record): k_speech_rec_* scratch, the packed records on the host
     bool speech_record = false, rec_ready = false; u64 rec_total = 0;
@@ -213,8 +234,6 @@ static int ensure_host(nutsb_ctx *c, HBuf &b, size_t bytes)
     b.cap = want;
     return NUTSB_OK;
 }
-static void release(DBuf &b) { if (b.p) cudaFree(b.p); b.p = nullptr; b.cap = 0; }
-static void release(HBuf &b) { if (b.p) cudaFreeHost(b.p); b.p = nullptr; b.cap = 0; }
 
 static int upload(nutsb_ctx *c, DBuf &b, const void *src, size_t bytes)
 {
@@ -293,10 +312,10 @@ static int run_scan(nutsb_ctx *c, In in, Out out, i64 n_upper, const u32 *n_dev)
     return NUTSB_OK;
 }
 
-// Stable LSD radix sort of (key, val) pairs.  On return *keys / *vals point at
-// the sorted arrays (one of the two ping-pong buffers).  vals start as iota.
+// Stable LSD radix sort of (key, val) pairs from kb[0] / vb[0].  On return *keys / *vals point at
+// the sorted arrays (one of the two ping-pong buffers).  vals start as iota unless vals_given.
 static int radix_sort(nutsb_ctx *c, DBuf kb[2], DBuf vb[2], i64 n_upper, const u32 *n_dev, u32 key_bits,
-                      u32 **keys, u32 **vals)
+                      u32 **keys, u32 **vals, bool vals_given = false)
 {
     const u32 passes = key_bits ? cdiv(key_bits, NUTSB_RS_BITS) : 1;
     const u32 bits = std::max(1u, cdiv(key_bits, passes));            // digit width: passes balanced, tables small
@@ -312,7 +331,7 @@ static int radix_sort(nutsb_ctx *c, DBuf kb[2], DBuf vb[2], i64 n_upper, const u
                      c->d_hist.as<u32>(), nblk); CKL();
         TRY(run_scan(c, InU32{c->d_hist.as<u32>()}, OutU64{c->d_hoffs.as<u64>()}, (i64)hn, nullptr));
         NUTSB_LAUNCH(nblk, NUTSB_RS_THREADS, c->stream, k_rs_scatter, kb[cur].as<u32>(),
-                     p == 0 ? (const u32 *)nullptr : vb[cur].as<u32>(), n_upper, n_dev, shift, bits,
+                     p == 0 && !vals_given ? (const u32 *)nullptr : vb[cur].as<u32>(), n_upper, n_dev, shift, bits,
                      c->d_hoffs.as<u64>(), nblk, kb[cur ^ 1].as<u32>(), vb[cur ^ 1].as<u32>()); CKL();
         c->tm.launches += 2;
         cur ^= 1;
@@ -485,34 +504,11 @@ NUTSB_API void nutsb_destroy(nutsb_ctx *c)
     if (!c) return;
     cudaSetDevice(c->device);
     if (c->stream) cudaStreamSynchronize(c->stream);
-    DBuf *all[] = { &c->d_codetab, &c->swear.trans, &c->swear.clsmap, &c->swear.tr16, &c->swear.cls2, &c->site.trans, &c->site.clsmap, &c->site.tr16, &c->site.cls2,
-        &c->userban.slot_off, &c->userban.slot_len, &c->userban.pool,
-        &c->d_user_room, &c->d_user_slot, &c->d_slot_user, &c->d_room_slot_off, &c->d_slot_cf, &c->d_slot_lv,
-        &c->cls[0].d_user_cls, &c->cls[0].d_room_cls_off, &c->cls[0].d_cls_flags, &c->cls[0].d_cls_level,
-        &c->cls[1].d_user_cls, &c->cls[1].d_room_cls_off, &c->cls[1].d_cls_flags, &c->cls[1].d_cls_level,
-        &c->d_status, &c->d_len_on, &c->d_len_off, &c->d_nrep, &c->d_eoff, &c->d_sums, &c->d_scan_ticket, &c->d_ek[0], &c->d_ek[1],
-        &c->d_ev_[0], &c->d_ev_[1], &c->d_hist, &c->d_hoffs, &c->d_room_ent_off, &c->d_e_info, &c->d_e_delta,
-        &c->d_e_slot, &c->d_e_scan, &c->d_counts, &c->d_room_b_off, &c->d_bl_op, &c->d_bl_room, &c->d_evk[0],
-        &c->d_evk[1], &c->d_evv[0], &c->d_evv[1], &c->d_ev_ukey, &c->d_ev_delta, &c->d_ev_op, &c->d_sv_ukey,
-        &c->d_sv_delta, &c->d_sv_op, &c->d_sv_pre, &c->d_ev_off, &c->d_vp_on, &c->d_vp_off, &c->d_cp,
-        &c->d_room_tile_off, &c->d_room_cell_off, &c->d_room_item_off, &c->d_sizes, &c->d_counters,
-        &c->d_runs, &c->d_slots, &c->d_items, &c->d_slab, &c->d_bl_meta, &c->d_off, &c->d_out, &c->d_digest, &c->d_ulen,
-        &c->d_dpre, &c->d_dir, &c->d_iov, &c->d_iov_first, &c->d_iov_cnt, &c->d_room_users, &c->d_room_users_off, &c->d_dg,
-        &c->s_text, &c->s_toff, &c->s_kind, &c->s_target, &c->s_except, &c->s_flags, &c->s_gate, &c->s_verdict, &c->s_v8,
-        &c->d_names, &c->d_name_off, &c->d_sflags, &c->d_lit, &c->d_lit_off, &c->d_sp_len, &c->d_sp_off, &c->d_sp_text,
-        &c->d_sp_kind, &c->d_sp_target, &c->d_sp_except, &c->d_sp_flags, &c->d_sp_gate, &c->d_sp_verdict,
-        &c->s_verb, &c->s_speaker, &c->s_body, &c->s_boff,
-        &c->d_g_user_shard, &c->d_g_user_local, &c->d_g_has_room, &c->d_g_names, &c->d_g_name_off, &c->d_g_sflags, &c->d_sp_keep, &c->d_sp_sel,
-        &c->d_rec_key, &c->d_rec_line, &c->d_rec_k[0], &c->d_rec_k[1], &c->d_rec_v[0], &c->d_rec_v[1], &c->d_rec_cnt, &c->d_rec_seg,
-        &c->d_rec_lens, &c->d_rec_bytes, &c->d_rec_off, &c->d_rec_out };
-    for (DBuf *b : all) release(*b);
-    release(c->h_small); release(c->h_off); release(c->h_out);
-    release(c->h_dir); release(c->h_iov); release(c->h_iov_first); release(c->h_iov_cnt); release(c->h_rec);
     for (auto &e : c->ev) if (e) cudaEventDestroy(e);
     for (auto &e : c->dep) if (e) cudaEventDestroy(e);
     if (c->side) { cudaStreamSynchronize(c->side); cudaStreamDestroy(c->side); }
     if (c->own_stream && c->stream) cudaStreamDestroy(c->stream);
-    delete c;
+    delete c;                                                   // (the buffers free themselves)
 }
 
 static int set_swear_impl(nutsb_ctx *c, const char *const *words)
@@ -554,7 +550,7 @@ NUTSB_API int nutsb_create(nutsb_ctx **out, int device)
         CK(cudaFuncSetAttribute(k_ac_pair<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, NUTSB_ACP_SMEM(2 * NUTSB_AC_SMEM_ENTRIES)));
         u8 tab[NUTSB_CODETAB_BYTES]; build_codetab(tab);
         TRY(upload(c, c->d_codetab, tab, sizeof tab));
-        TRY(ensure(c, c->d_status, 64)); TRY(ensure(c, c->d_counts, 64)); TRY(ensure(c, c->d_sizes, sizeof(Sizes)));
+        TRY(ensure(c, c->d_status, 64)); TRY(ensure(c, c->d_counts, 64));
         TRY(ensure(c, c->d_counters, 1024));
         TRY(ensure_host(c, c->h_small, 4096));
         {   // the callers' literals (nutsb_speech.cuh)
@@ -734,10 +730,10 @@ static int set_users_impl(nutsb_ctx *c, int32_t n_users, int32_t n_rooms, const 
     // create_user c:2747 and clear_revbuff c:2626 only): room r keeps buffer r; user u keeps the buffer of
     // prev_index[u] (nutsb_set_users_remap), index u itself without a map; new rooms / users start empty
     {
-        std::vector<nutsb_ctx::RevBuf> rev((size_t)n_rooms, nutsb_ctx::RevBuf{});
+        std::vector<ReviewRing<NUTSB_REVIEW_LINES>> rev((size_t)n_rooms, ReviewRing<NUTSB_REVIEW_LINES>{});
         for (size_t r = 0; r < rev.size() && r < c->rev.size(); ++r) rev[r] = c->rev[r];
         c->rev.swap(rev);
-        std::vector<nutsb_ctx::TellBuf> rt((size_t)n_users, nutsb_ctx::TellBuf{});
+        std::vector<ReviewRing<NUTSB_REVTELL_LINES>> rt((size_t)n_users, ReviewRing<NUTSB_REVTELL_LINES>{});
         for (i32 u = 0; u < n_users; ++u) {
             const i32 p = prev_index ? prev_index[u] : u;
             if (p >= 0 && (size_t)p < c->revtell.size()) rt[(size_t)u] = c->revtell[(size_t)p];
@@ -1064,26 +1060,9 @@ static int run_write(nutsb_ctx *c, const nutsb_ops *o, nutsb_streams *out, IovRe
     for (int q = 0; q < 2; ++q) { TRY(ensure(c, c->d_ek[q], (size_t)E * 4 + 16)); TRY(ensure(c, c->d_ev_[q], (size_t)E * 4 + 16)); }
     NUTSB_LAUNCH(cdiv(n, 256), 256, st, k_expand, ops, pop, nrep, c->d_eoff.as<u64>(), c->d_ek[0].as<u32>(), c->d_ev_[0].as<u32>()); CKL();
     c->tm.launches++;
-    // the op index rides as the key's payload: first pass must not use iota
+    // the op index rides as the key's payload: the first pass must not use iota
     u32 *e_room = nullptr, *e_op = nullptr;
-    {
-        const u32 kbits = std::max(1u, bits_for((u64)Rt));
-        const u32 passes = cdiv(kbits, NUTSB_RS_BITS);
-        const u32 bits = cdiv(kbits, passes);
-        const u32 nblk = cdiv(E, NUTSB_RS_CHUNK);
-        const size_t hn = ((size_t)1 << bits) * nblk;
-        TRY(ensure(c, c->d_hist, hn * 4)); TRY(ensure(c, c->d_hoffs, (hn + 1) * 8));
-        int cur = 0;
-        for (u32 p = 0; p < passes; ++p) {
-            const int shift = (int)(p * bits);
-            NUTSB_LAUNCH(nblk, NUTSB_RS_THREADS, st, k_rs_hist, c->d_ek[cur].as<u32>(), (i64)E, (const u32 *)nullptr, shift, bits, c->d_hist.as<u32>(), nblk); CKL();
-            TRY(run_scan(c, InU32{c->d_hist.as<u32>()}, OutU64{c->d_hoffs.as<u64>()}, (i64)hn, nullptr));
-            NUTSB_LAUNCH(nblk, NUTSB_RS_THREADS, st, k_rs_scatter, c->d_ek[cur].as<u32>(), c->d_ev_[cur].as<u32>(), (i64)E,
-                         (const u32 *)nullptr, shift, bits, c->d_hoffs.as<u64>(), nblk, c->d_ek[cur ^ 1].as<u32>(), c->d_ev_[cur ^ 1].as<u32>()); CKL();
-            c->tm.launches += 2; cur ^= 1;
-        }
-        e_room = c->d_ek[cur].as<u32>(); e_op = c->d_ev_[cur].as<u32>();
-    }
+    TRY(radix_sort(c, c->d_ek, c->d_ev_, (i64)E, nullptr, std::max(1u, bits_for((u64)Rt)), &e_room, &e_op, true));
     TRY(ensure(c, c->d_room_ent_off, ((size_t)Rt + 2) * 4));
 
     // -- C. classify entries, scatter the slab list and the event list
@@ -1765,15 +1744,11 @@ NUTSB_API int nutsb_q_more(nutsb_ctx *c, int32_t user, int32_t sock_user, const 
 
 NUTSB_API int64_t nutsb_q_pending(const nutsb_ctx *c) { return c ? (int64_t)c->q.n() : 0; }
 
-// record(), nuts333.c:2062-2071: strncpy pads with NULs, byte REVIEW_LEN becomes '\n', the next one NUL.
+// record(), nuts333.c:2062-2071
 static void do_record(nutsb_ctx *c, i32 room, const char *str)
 {
     if (room < 0 || room >= (i32)c->rev.size()) return;
-    nutsb_ctx::RevBuf &rb = c->rev[(size_t)room];
-    strncpy(rb.buf[rb.line], str, NUTSB_REVIEW_LEN);
-    rb.buf[rb.line][NUTSB_REVIEW_LEN] = '\n';
-    rb.buf[rb.line][NUTSB_REVIEW_LEN + 1] = '\0';
-    rb.line = (rb.line + 1) % NUTSB_REVIEW_LINES;
+    c->rev[(size_t)room].put(str, strnlen(str, NUTSB_REVIEW_LEN));
 }
 
 // The swear verdicts of the queued lines, taken in one device batch.
@@ -1823,7 +1798,7 @@ NUTSB_API int nutsb_q_review(nutsb_ctx *c, int32_t user, int32_t room, const cha
     if (!c || !room_name) return NUTSB_E_INVAL;
     if (room < 0 || room >= c->R) return fail(c, NUTSB_E_RANGE, "room index out of range%s");
     TRY(resolve_records(c));
-    const nutsb_ctx::RevBuf &rb = c->rev[(size_t)room];
+    const auto &rb = c->rev[(size_t)room];
     int cnt = 0;
     for (int i = 0; i < NUTSB_REVIEW_LINES; ++i) {
         const int line = (rb.line + i) % NUTSB_REVIEW_LINES;
@@ -1968,11 +1943,7 @@ static std::string user_name(const nutsb_ctx *c, i32 u)
 
 static void do_record_tell(nutsb_ctx *c, i32 u, const char *str)     // record_tell(), c:2074
 {
-    nutsb_ctx::TellBuf &rb = c->revtell[(size_t)u];
-    strncpy(rb.buf[rb.line], str, NUTSB_REVIEW_LEN);
-    rb.buf[rb.line][NUTSB_REVIEW_LEN] = '\n';
-    rb.buf[rb.line][NUTSB_REVIEW_LEN + 1] = '\0';
-    rb.line = (rb.line + 1) % NUTSB_REVTELL_LINES;
+    c->revtell[(size_t)u].put(str, strnlen(str, NUTSB_REVIEW_LEN));
 }
 
 static int q_private(nutsb_ctx *c, int pemote, i32 user, i32 target, const char *inpstr)
@@ -2042,7 +2013,7 @@ NUTSB_API int nutsb_q_revtell(nutsb_ctx *c, int32_t user)
 {
     if (!c) return NUTSB_E_INVAL;
     if (user < 0 || user >= c->U || (size_t)user >= c->revtell.size()) return fail(c, NUTSB_E_RANGE, "user index out of range%s");
-    const nutsb_ctx::TellBuf &rb = c->revtell[(size_t)user];
+    const auto &rb = c->revtell[(size_t)user];
     int cnt = 0;
     for (int i = 0; i < NUTSB_REVTELL_LINES; ++i) {
         const int line = (rb.line + i) % NUTSB_REVTELL_LINES;
@@ -2104,7 +2075,7 @@ static int fetch_records(nutsb_ctx *c)
 }
 
 // ... and into the rings: room r's c records end at (line + c) % REVIEW_LINES, the last min(c, REVIEW_LINES) of them
-// where record() would have put them (do_record: strncpy's NUL padding, '\n' at REVIEW_LEN).
+// where record() would have put them.
 static void apply_records(nutsb_ctx *c)
 {
     const u8 *p = c->h_rec.as<u8>(), *end = p + c->rec_total;
@@ -2114,15 +2085,9 @@ static void apply_records(nutsb_ctx *c)
         const u8 *lens = p + 8;
         const u32 t = std::min<u32>(cnt, NUTSB_REVIEW_LINES);
         const u8 *text = p + NUTSB_REC_HEAD;
-        nutsb_ctx::RevBuf &rb = c->rev[room];
-        for (u32 i = 0; i < t; ++i) {
-            char *row = rb.buf[(rb.line + (cnt - t) + i) % NUTSB_REVIEW_LINES];
-            memset(row, 0, NUTSB_REVIEW_LEN);
-            memcpy(row, text, lens[i]);
-            row[NUTSB_REVIEW_LEN] = '\n'; row[NUTSB_REVIEW_LEN + 1] = '\0';
-            text += lens[i];
-        }
-        rb.line = (int)((rb.line + cnt) % NUTSB_REVIEW_LINES);
+        auto &rb = c->rev[room];
+        rb.line = (int)((rb.line + (cnt - t)) % NUTSB_REVIEW_LINES);
+        for (u32 i = 0; i < t; ++i) { rb.put(text, lens[i]); text += lens[i]; }
         p = text;
     }
     c->rec_ready = false;
@@ -2134,7 +2099,7 @@ NUTSB_API int nutsb_get_review_buffer(nutsb_ctx *c, int32_t room, uint8_t *rows,
 {
     if (!c) return NUTSB_E_INVAL;
     if (room < 0 || room >= (i32)c->rev.size()) return fail(c, NUTSB_E_RANGE, "room index out of range%s");
-    const nutsb_ctx::RevBuf &rb = c->rev[(size_t)room];
+    const auto &rb = c->rev[(size_t)room];
     if (rows) memcpy(rows, rb.buf, sizeof rb.buf);
     if (line) *line = rb.line;
     return NUTSB_OK;

@@ -49,7 +49,7 @@ struct nutsb_multi {
     std::vector<u64> dg_local;
     // every room's review buffer in global order, taken from the last plan that was set up whole, until a re-plan
     // succeeds (one that fails half way has already reshaped some shards' buffers: its retry starts from these)
-    std::vector<nutsb_ctx::RevBuf> rev_carry; bool carry = false;
+    std::vector<ReviewRing<NUTSB_REVIEW_LINES>> rev_carry; bool carry = false;
 };
 
 static int mfail(nutsb_multi *m, int code, const char *msg) { if (m) m->err = msg; return code; }
@@ -189,7 +189,7 @@ NUTSB_API int nutsb_multi_set_users(nutsb_multi *m, int32_t n_users, int32_t n_r
     // every room's review buffer as the old plan holds it (on a shard this process runs), to follow the room to its
     // new shard and local index; a room new to the population starts empty, as on one context
     if (m->have_users) {
-        m->rev_carry.assign((size_t)m->R, nutsb_ctx::RevBuf{});
+        m->rev_carry.assign((size_t)m->R, ReviewRing<NUTSB_REVIEW_LINES>{});
         for (i32 r = 0; r < m->R; ++r) {
             const nutsb_ctx *c = m->ctx[(size_t)m->room_shard[(size_t)r]];
             const size_t l = (size_t)m->room_local[(size_t)r];
@@ -239,7 +239,7 @@ NUTSB_API int nutsb_multi_set_users(nutsb_multi *m, int32_t n_users, int32_t n_r
     }
     for (i32 r = 0; r < n_rooms; ++r)
         if (nutsb_ctx *c = m->ctx[(size_t)m->room_shard[(size_t)r]])
-            c->rev[(size_t)m->room_local[(size_t)r]] = m->carry && (size_t)r < m->rev_carry.size() ? m->rev_carry[(size_t)r] : nutsb_ctx::RevBuf{};
+            c->rev[(size_t)m->room_local[(size_t)r]] = m->carry && (size_t)r < m->rev_carry.size() ? m->rev_carry[(size_t)r] : ReviewRing<NUTSB_REVIEW_LINES>{};
     m->rev_carry.clear(); m->carry = false;
     m->len.assign((size_t)n_users, 0); m->ptr.assign((size_t)n_users, nullptr);
     m->iov.assign((size_t)n_users, nullptr); m->count.assign((size_t)n_users, 0);

@@ -12,15 +12,19 @@ from pathlib import Path
 
 HERE = Path(__file__).resolve().parent
 ROOT = HERE.parent.parent
+if str(ROOT) not in sys.path:                 # (run as a script)
+    sys.path.insert(0, str(ROOT))
+from nuts333_b200.build import HEADERS, SOURCES  # noqa: E402
+
 CSRC = ROOT / "nuts333_b200" / "csrc"
 OUT = HERE / "_build" / "libnutsb200_sim.so"
+# the product library's own sources and headers: an edit to any of them rebuilds the emulated one too
+DEPS = SOURCES + HEADERS + [HERE / "cpusim.h", Path(__file__).resolve()]
 
 
 def build_sim(force: bool = False, sanitize: str | None = None) -> Path:
     out = OUT if not sanitize else OUT.with_name(f"libnutsb200_sim_{sanitize}.so")
-    deps = [CSRC / f for f in ("nutsb_lib.cu", "nutsb_common.cuh", "nutsb_kernels.cuh", "nutsb_match.cuh")]
-    deps += [HERE / "cpusim.h", ROOT / "include" / "nutsb200.h", Path(__file__)]
-    if not force and out.exists() and all(d.stat().st_mtime <= out.stat().st_mtime for d in deps):
+    if not force and out.exists() and all(d.stat().st_mtime <= out.stat().st_mtime for d in DEPS):
         return out
     out.parent.mkdir(parents=True, exist_ok=True)
     cmd = ["g++", "-std=c++17", "-O1", "-g", "-fPIC", "-shared", "-pthread", "-DNUTSB_CPUSIM",
